@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- proving throughput of the state-transition AIR (BASELINE.json: "prove ms & tx/s, state-transition AIR").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--num-tx T] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--num-tx T] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one complete proof (Prover::prove, /root/reference/src/lib.rs:140) of one synthetic batch of T transactions
 (default 1024: trace 2^20 rows x 94 columns, blowup 8 -> 2^23 LDE rows; BASELINE.json configs[3]).  With N > 1 (launched
@@ -18,6 +18,8 @@ data-path collective, scaling is weak -- that is `value`.  The same run then als
   cpu_baseline  the CPU oracle (a port: the Rust reference cannot be built here) proving the SAME batch once, N=1 rank 0 only;
             its proof bytes are compared with the GPU's (`parity`)
 --impl reference times that CPU port alone, with all host threads, on full-size batches.
+--dump-outputs DIR writes the proof of the last timed step, one float32 value per byte, to DIR/proof.npy (DIR/proof_rank<r>.npy
+with N > 1): the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -32,6 +34,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True       # the tree may be read-only: no __pycache__ of the modules imported below
 
 METRIC, UNIT = "state_transition_prove_throughput", "tx/s"
 TRACE_WIDTH, ROWS_PER_TX, BLOWUP = 94, 1024, 8
@@ -185,6 +188,11 @@ def cpu_port_run(num_tx, steps, warmup, seed=1, want_proof=False):
     return (sec, proof) if want_proof else sec
 
 
+def dump_proof(directory, name, proof):
+    """--dump-outputs: proof bytes as float32 (exact for 0..255)"""
+    np.save(Path(directory) / f"{name}.npy", np.frombuffer(proof, dtype=np.uint8).astype(np.float32))
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference path's CPU implementation.  The reference is Rust over an un-vendored winterfell fork
     and no Rust toolchain exists in this image, so what runs is the C/OpenMP port of that path (oracle/) with all host threads,
@@ -196,7 +204,10 @@ def run_reference(args, rank, world):
     budget_s, times = float(os.environ.get("CSG_REFERENCE_BUDGET_S", "150")), []
     t_all = time.perf_counter()
     while len(times) < max(args.steps, 1) and (not times or time.perf_counter() - t_all + times[-1] <= budget_s):
-        times.append(cpu_port_run(args.num_tx, 1, 0, seed=1000))
+        sec, proof = cpu_port_run(args.num_tx, 1, 0, seed=1000, want_proof=True)
+        times.append(sec)
+    if args.dump_outputs:
+        dump_proof(args.dump_outputs, "proof", proof)
     sec = sum(times) / len(times)
     value = args.num_tx / sec
     cores = os.cpu_count() or 1
@@ -229,7 +240,12 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile", action="store_true", help="short run for ncu: 1 warm-up, no e2e leg, no CPU baseline (not a bench number)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the proof of the last timed step to DIR/proof.npy (float32, one value per byte)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)      # a bad path fails before the timed work, not after it
     rank, world, local_rank = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     # torchrun pins OMP_NUM_THREADS=1; the host-side witness builder and the CPU port are OpenMP code: give them the cores
     # (the reference arm runs on rank 0 alone and takes all of them)
@@ -299,6 +315,8 @@ def main():
         barrier()
         wall_ms = (time.perf_counter() - t0) * 1e3
     clock_summary = clocks.summary()
+    if args.dump_outputs:
+        dump_proof(args.dump_outputs, "proof" if world == 1 else f"proof_rank{rank}", p)
 
     # ---- timed region 2: end to end through the C ABI with host buffers (a) page-locked, (b) pageable
     e2e_ms, e2e_h2d_ms, e2e_pg_ms, e2e_pipe_ms = 0.0, 0.0, 0.0, 0.0

@@ -16,9 +16,9 @@ What it restates, each from the reference file it cites (paths relative to /root
   * the batch metadata of TransactionMetadata::build_random src/lib.rs:235-464 (own PRNG; keys by the SURVEY.md 8(d) recipe)
 
 Constants (MDS, INV_MDS, ARK, GENERATOR, B3) come from this module's OWN parse of src/utils/rescue.rs:385-996 and
-src/utils/ecc.rs:23-45 (`parse_reference_constants`), not from tools/gen_constants.py.  The parse is stored in
-tests/golden/air_constants.json by tests/golden/make_air_vectors.py so that the module also runs where /root/reference does not
-exist (the GPU box).  Only tests/ and tests/golden/make_air_vectors.py import this file.
+src/utils/ecc.rs:23-45 (`parse_reference_constants`), not from tools/gen_constants.py.  tests/golden/make_air_vectors.py
+stores the parse in tests/golden/air_constants.json, and the module reads it from there: it runs without the reference
+sources.  Only tests/ and tests/golden/make_air_vectors.py import this file.
 """
 import json
 import re
@@ -29,7 +29,6 @@ R_MONT = (1 << 64) % P            # BaseElement::from_raw_unchecked values are M
 INV_ALPHA = 3146514939656186539   # src/utils/rescue.rs:383
 HERE = Path(__file__).resolve().parent
 CONSTANTS_JSON = HERE.parent / "tests" / "golden" / "air_constants.json"
-REFERENCE = Path("/root/reference")
 
 STATE, RATE, ROUNDS, CYCLE = 14, 7, 7, 8     # src/utils/rescue.rs:25-37
 COORD, AFFINE, PROJ = 6, 12, 18              # src/utils/ecc.rs:16-20
@@ -49,7 +48,8 @@ def _const_block(text, name):
     return text[m.end():i - 1]
 
 
-def parse_reference_constants(root=REFERENCE):
+def parse_reference_constants(root):
+    """the constant tables of a checkout of the reference at `root`"""
     rescue = (root / "src/utils/rescue.rs").read_text()
     ecc = (root / "src/utils/ecc.rs").read_text()
     mds, inv_mds = _numbers(_const_block(rescue, "MDS")), _numbers(_const_block(rescue, "INV_MDS"))
@@ -63,13 +63,7 @@ def parse_reference_constants(root=REFERENCE):
     return {"MDS": mds, "INV_MDS": inv_mds, "ARK": ark, "GENERATOR": [g * rinv % P for g in gen_raw], "B3": b3}
 
 
-def load_constants():
-    if (REFERENCE / "src/utils/rescue.rs").exists():
-        return parse_reference_constants()
-    return json.loads(CONSTANTS_JSON.read_text())
-
-
-_K = load_constants()
+_K = json.loads(CONSTANTS_JSON.read_text())
 MDS = [_K["MDS"][i * 14:(i + 1) * 14] for i in range(14)]
 INV_MDS = [_K["INV_MDS"][i * 14:(i + 1) * 14] for i in range(14)]
 ARK = [_K["ARK"][i * 28:(i + 1) * 28] for i in range(8)]

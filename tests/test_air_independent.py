@@ -7,6 +7,7 @@ tests/golden/air_vectors.txt holds, for all six AIRs: degrees, periodic-column f
 vectors of evaluate_transition on witness rows (all zero) and random frames (dense).  tests/host_harness.cpp checks oracle/airs.c
 slot by slot and the product's fused evaluation through random linear combinations of the golden slots."""
 import json
+import re
 import subprocess
 from pathlib import Path
 
@@ -51,14 +52,25 @@ def test_the_golden_check_notices_a_wrong_slot(harness, tmp_path):
     assert out.returncode != 0 and "oracle/airs.c result[59] differs" in out.stdout and "product airs.cuh merged value differs" in out.stdout
 
 
+def header_tables(text):
+    """name -> values of the uint64 tables of a header written by tools/gen_constants.py (`NAME[n] = {...};` or `#define NAME_VALUES`)"""
+    blocks = re.findall(r"(?:uint64_t (\w+)\[\d+\] = \{|#define (\w+)_VALUES)(.*?)(?:\};|\n(?!\s+0x))", text, re.S)
+    return {a or b: [int(v, 16) for v in re.findall(r"0x([0-9a-f]{16})ULL", body)] for a, b, body in blocks}
+
+
 def test_pyair_constants_are_its_own_parse_of_the_reference(pyair):
+    # pyair's stored parse of the reference (tests/golden/make_air_vectors.py) is what it runs on, and it agrees with the tables
+    # tools/gen_constants.py parsed separately from the same sources for the C oracle (canonical) and the product (Montgomery)
+    names = ("MDS", "INV_MDS", "ARK", "GENERATOR", "B3")
     stored = json.loads((ROOT / "tests" / "golden" / "air_constants.json").read_text())
-    if not (pyair.REFERENCE / "src/utils/rescue.rs").exists():
-        pytest.skip("/root/reference is not present on this box: the stored parse is what pyair runs on")
-    parsed = pyair.parse_reference_constants()
-    assert all(stored[k] == parsed[k] for k in ("MDS", "INV_MDS", "ARK", "GENERATOR", "B3"))
-    # and they agree with what the C oracle / the product were generated with (tools/gen_constants.py): MDS * INV_MDS = I, generator on the curve
+    assert [pyair._K[k] for k in names] == [stored[k] for k in names]
     P = pyair.P
+    oracle_h = header_tables((ROOT / "oracle" / "ref_constants.h").read_text())
+    product_h = header_tables((ROOT / "certificate_stark_b200" / "csrc" / "ref_constants.h").read_text())
+    for k in names:
+        assert oracle_h["REF_" + k] == stored[k], k
+        assert product_h["CSG_" + k] == [v * 2**64 % P for v in stored[k]], k
+    # MDS * INV_MDS = I, generator on the curve
     assert all(sum(pyair.MDS[i][k] * pyair.INV_MDS[k][j] for k in range(14)) % P == (1 if i == j else 0) for i in range(14) for j in range(14))
     gx, gy = pyair.GENERATOR[0:6], pyair.GENERATOR[6:12]
     b = [v * pow(3, -1, P) % P for v in pyair.B3]

@@ -5,6 +5,7 @@ import ctypes as C
 import os
 import re
 import subprocess
+import sys
 from pathlib import Path
 
 import numpy as np
@@ -39,15 +40,28 @@ def test_ctypes_mirrors_match_the_header_layout(csg, tmp_path):
     assert csg.Timings.stage_launches.offset == off_stage
 
 
+NO_DEVICE = r"""
+import sys
+sys.path.insert(0, sys.argv[1])
+import certificate_stark_b200 as csg
+for make in (lambda: csg.Context(0), lambda: csg.get_example(2)):
+    try:
+        make()
+    except csg.CsgError as e:
+        print(e)
+    else:
+        raise SystemExit("created without a CUDA device")
+assert b"no context" in csg.lib().csg_last_error(None)
+"""
+
+
 def test_no_cpu_fallback(csg):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    with pytest.raises(csg.CsgError, match="no CPU fallback"):
-        csg.Context(0)
-    with pytest.raises(csg.CsgError):
-        csg.get_example(2)
-    assert b"no context" in csg.lib().csg_last_error(None)
+    # with no CUDA device visible (hidden from a child process, so that this also runs on a machine with a GPU) every entry
+    # point raises instead of computing on the CPU
+    out = subprocess.run([sys.executable, "-c", NO_DEVICE, str(ROOT)], capture_output=True, text=True,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert out.returncode == 0, (out.stdout + out.stderr)[-2000:]
+    assert "no CPU fallback" in out.stdout.splitlines()[0]
 
 
 def test_host_harness_against_oracle(oracle, tmp_path):
