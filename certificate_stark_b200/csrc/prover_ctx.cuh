@@ -258,6 +258,14 @@ struct csg_ctx {
             // (the Schnorr AIR's periodic columns carry the public keys and messages: those tables follow the public inputs)
             same_periodic = same_periodic && fresh.periodic.size() == air.periodic.size();
             for (size_t c = 0; same_periodic && c < fresh.periodic.size(); c++) same_periodic = fresh.periodic[c].values == air.periodic[c].values;
+            if (!(same_shape && same_periodic)) {
+                // From here on the members describe the new shape while the device tables still hold the old one, and any
+                // check below may throw: until this call completes the context has no AIR, so a repeated call with the same
+                // arguments cannot take the fast path above, and no proof runs on the mixed state.  A prefetched trace of the
+                // old shape is dropped.
+                stage = S_NONE;
+                if (next_pending) { CSG_CUDA(cudaStreamSynchronize(copy_stream)); next_pending = false; }
+            }
             air = std::move(fresh);
         }
         if (same_shape && same_periodic) {
@@ -301,7 +309,6 @@ struct csg_ctx {
         build_periodic_tables();
         lde_tables.build(lde_shift.data(), bl, logn, st);
         nfri = 0;
-        if (next_pending) { CSG_CUDA(cudaStreamSynchronize(copy_stream)); next_pending = false; }   // a prefetched trace of another shape is dropped
         stage = S_AIR;
     }
 

@@ -57,13 +57,24 @@ def hash_elements(vals):
 @pytest.mark.parametrize("ext", [1, 2, 3])
 @pytest.mark.parametrize("kind", ["rescue", "transaction"])
 def test_stage_calls_with_external_transcript_reproduce_csg_prove(ctx, csg, kind, ext):
-    L = csg.lib()
     if kind == "rescue":
-        air, blowup, ncons, nassert, ce = csg.AIR_RESCUE, 4, 14, 14, 4
         trace, pub = csg.build_rescue_trace(np.arange(42, 49, dtype=np.uint64), 64)
+        stage_calls_reproduce_csg_prove(ctx, csg, csg.AIR_RESCUE, trace, pub, 4, ext, ncons=14, nassert=14, ce=4)
     else:
-        air, blowup, ncons, nassert, ce = csg.AIR_TRANSACTION, 8, 115, 4, 8
         trace, pub = csg.TransactionBatch(seed=6, num_tx=1).transaction_trace()
+        stage_calls_reproduce_csg_prove(ctx, csg, csg.AIR_TRANSACTION, trace, pub, 8, ext, ncons=115, nassert=4, ce=8)
+
+
+@pytest.mark.parametrize("num_tx,ext", [(16, 1), (16, 3), (2048, 1)])
+def test_transaction_stage_calls_at_size_reproduce_csg_prove(ctx, csg, num_tx, ext):
+    # 16 transactions (2^14 rows): csg_eval_constraints takes the low-degree split, with E-valued coefficients at ext 3;
+    # 2048 transactions (2^21 rows): the 1024-point NTT passes.  test_gpu_headline.py pins csg_prove at this shape to the oracle.
+    trace, pub = csg.TransactionBatch(seed=6, num_tx=num_tx).transaction_trace()
+    stage_calls_reproduce_csg_prove(ctx, csg, csg.AIR_TRANSACTION, trace, pub, 8, ext, ncons=115, nassert=4, ce=8)
+
+
+def stage_calls_reproduce_csg_prove(ctx, csg, air, trace, pub, blowup, ext, ncons, nassert, ce):
+    L = csg.lib()
     opt = csg.ProofOptions(blowup_factor=blowup, field_extension=ext)
     want = ctx.prove(air, trace, pub, opt)
     flat = lambda elems: [w_ for e in elems for w_ in e]      # an element of E crosses the ABI as its `ext` words in order

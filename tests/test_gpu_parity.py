@@ -131,7 +131,7 @@ def test_merkle_init_proof_identical_to_oracle(ctx, oracle, csg):
         assert oracle.verify(oracle.AIR_MERKLE_INIT, pub, got) == 0
 
 
-@pytest.mark.parametrize("num_tx", [1, 2, 16])
+@pytest.mark.parametrize("num_tx", [1, 2, 16, 128])     # 128: the largest batch of benches/merkle.rs
 def test_merkle_update_proof_identical_to_oracle(ctx, oracle, csg, num_tx):
     batch = csg.TransactionBatch(seed=3, num_tx=num_tx)
     trace, pub = batch.merkle_update_trace()
@@ -140,7 +140,7 @@ def test_merkle_update_proof_identical_to_oracle(ctx, oracle, csg, num_tx):
     assert oracle.verify(oracle.AIR_MERKLE_UPDATE, pub, got) == 0
 
 
-@pytest.mark.parametrize("num_sig", [1, 2, 8])
+@pytest.mark.parametrize("num_sig", [1, 2, 8, 32, 128])   # from 32 signatures (2^14 rows) on the low-degree split runs; 128: benches/schnorr.rs
 def test_schnorr_proof_identical_to_oracle(ctx, oracle, csg, num_sig):
     batch = csg.SignatureBatch(seed=5, num_sig=num_sig)
     trace, pub = batch.schnorr_trace()
@@ -149,7 +149,7 @@ def test_schnorr_proof_identical_to_oracle(ctx, oracle, csg, num_sig):
     assert oracle.verify(oracle.AIR_SCHNORR, pub, got) == 0
 
 
-@pytest.mark.parametrize("num_tx,hash_fn", [(1, 2), (4, 2), (2, 3), (16, 2)])
+@pytest.mark.parametrize("num_tx,hash_fn", [(1, 2), (4, 2), (2, 3), (16, 2), (128, 3)])
 def test_transaction_proof_identical_to_oracle(ctx, oracle, csg, num_tx, hash_fn):
     # config 1: the state-transition example at its smallest batches, default options (src/lib.rs:78-86)
     batch = csg.TransactionBatch(seed=1, num_tx=num_tx)
@@ -282,6 +282,74 @@ def test_errors_are_reported_not_swallowed(ctx, csg):
         batch = csg.TransactionBatch(seed=1, num_tx=1)
         t, p = batch.transaction_trace()
         ctx.prove(csg.AIR_TRANSACTION, t, p, csg.ProofOptions(blowup_factor=4))
+
+
+def test_rejected_set_air_is_rejected_again(csg, oracle):
+    # csg_set_air with the AIR, length and options of the last successful call keeps the device tables (the fast path of
+    # test_batch_after_batch_of_one_shape).  A call that fails on a check after the context's members took the new shape must
+    # not make the same arguments look like the last good shape: repeated, it has to fail again, with the same message, and
+    # the prove and prefetch calls must refuse to run on what it left.  The repeated set_air comes first: a context that took
+    # the fast path here would hold the tables of the old shape.
+    L = csg.lib()
+    rescue = lambda chain: csg.build_rescue_trace(np.arange(42, 49, dtype=np.uint64), chain)     # noqa: E731
+    r_trace, r_pub = rescue(32)                                                                   # 256 rows
+    tx_trace, tx_pub = csg.TransactionBatch(seed=1, num_tx=1).transaction_trace()
+    cases = [("constraint evaluation blowup", csg.AIR_TRANSACTION, tx_trace.shape[1], tx_pub, csg.ProofOptions(blowup_factor=4), tx_trace),
+             ("above 2^22", csg.AIR_RESCUE, 1 << 23, r_pub, csg.ProofOptions(), None),
+             ("FRI remainder", csg.AIR_RESCUE, r_trace.shape[1], r_pub, csg.ProofOptions(blowup_factor=32, fri_max_remainder_size=4), r_trace)]
+
+    def rejected_twice(c, air, n, pub, opt):
+        msgs = []
+        for _ in range(2):
+            with pytest.raises(csg.CsgError) as e:
+                c.set_air(air, n, pub, opt)
+            msgs.append((str(e.value), L.csg_last_error(c._h)))
+        assert msgs[0] == msgs[1]
+        return msgs[0][0]
+
+    with csg.Context(0) as c:
+        good = csg.ProofOptions(blowup_factor=4)
+        for reason, air, n, pub, opt, trace in cases:
+            c.set_air(csg.AIR_RESCUE, r_trace.shape[1], r_pub, good)          # a good shape first: the fast path is armed
+            assert reason in rejected_twice(c, air, n, pub, opt)
+            with pytest.raises(csg.CsgError):
+                c.prove_loaded()
+            with pytest.raises(csg.CsgError):
+                c.reload_resident_trace()
+            if trace is not None:
+                for _ in range(2):
+                    with pytest.raises(csg.CsgError):
+                        c.prove(air, trace, pub, opt)
+        # a prefetched trace does not survive a rejected set_air
+        hb = csg.HostBuffer(14, r_trace.shape[1])
+        try:
+            hb.array[:] = r_trace
+            c.set_air(csg.AIR_RESCUE, r_trace.shape[1], r_pub, good)
+            c.prefetch_trace_ptr(hb.ptr)
+            with pytest.raises(csg.CsgError):
+                c.set_air(csg.AIR_RESCUE, r_trace.shape[1], r_pub, csg.ProofOptions(blowup_factor=32, fri_max_remainder_size=4))
+            with pytest.raises(csg.CsgError):
+                c.prove_prefetched_ptr()
+            with pytest.raises(csg.CsgError):
+                c.set_air(csg.AIR_RESCUE, r_trace.shape[1], r_pub, csg.ProofOptions(blowup_factor=32, fri_max_remainder_size=4))
+            # and the context proves correctly afterwards, for the last good shape and for the others
+            c.set_air(csg.AIR_RESCUE, r_trace.shape[1], r_pub, good)
+            c.prefetch_trace_ptr(hb.ptr)
+            want = oracle.prove(oracle.AIR_RESCUE, r_trace, r_pub, oracle.options(blowup=4))
+            assert c.prove_prefetched_ptr() == want
+        finally:
+            hb.close()
+        assert c.prove(csg.AIR_RESCUE, r_trace, r_pub, good) == want
+        assert c.prove(csg.AIR_TRANSACTION, tx_trace, tx_pub, csg.ProofOptions()) == oracle.prove(oracle.AIR_TRANSACTION, tx_trace, tx_pub, oracle.options())
+    # the shard plan: 8 ranks cannot share the 4 LDE cosets of blowup 4.  One rank's set_air runs no collective.
+    with csg.LocalGroup(8) as grp:
+        r0 = grp.ctxs[0]
+        r0.set_air(csg.AIR_RESCUE, r_trace.shape[1], r_pub, csg.ProofOptions())
+        assert "divide the blowup" in rejected_twice(r0, csg.AIR_RESCUE, r_trace.shape[1], r_pub, good)
+        with pytest.raises(csg.CsgError):
+            r0.prove_loaded()
+        proofs = grp.prove(csg.AIR_RESCUE, r_trace, r_pub, csg.ProofOptions())
+    assert proofs == [oracle.prove(oracle.AIR_RESCUE, r_trace, r_pub, oracle.options())] * 8
 
 
 def test_device_field_arithmetic_selftest(ctx, csg):
