@@ -84,6 +84,7 @@ def lib() -> C.CDLL:
     sig = {
         "csg_create": (vp, [C.c_int]), "csg_destroy": (None, [vp]), "csg_last_error": (C.c_char_p, [vp]), "csg_free": (None, [vp]),
         "csg_prove": (C.c_int, [vp, C.c_int, _u64p, C.c_int, C.c_size_t, _u64p, C.c_size_t, opt, C.POINTER(_u8p), _szp]),
+        "csg_prove_many": (C.c_int, [vp, C.c_int, C.c_size_t, C.POINTER(_u64p), C.c_int, C.c_size_t, _u64p, C.c_size_t, opt, C.POINTER(_u8p), _szp]),
         "csg_prove_columns": (C.c_int, [vp, C.c_int, C.POINTER(_u64p), C.c_int, C.c_size_t, _u64p, C.c_size_t, opt, C.POINTER(_u8p), _szp]),
         "csg_set_air": (C.c_int, [vp, C.c_int, C.c_size_t, opt, _u64p, C.c_size_t]),
         "csg_load_trace": (C.c_int, [vp, _u64p, C.c_int]), "csg_reload_resident_trace": (C.c_int, [vp]),
@@ -226,6 +227,26 @@ class Context:
         out, n = _u8p(), C.c_size_t()
         self._check(lib().csg_prove(self._h, air_id, _p64(trace), repr, trace.shape[1], _p64(pub), pub.size, C.byref(options), C.byref(out), C.byref(n)))
         return self._take_proof(out, n)
+
+    def prove_many(self, air_id: int, traces, pubs, options: ProofOptions, repr: int = REPR_CANONICAL) -> list:
+        """csg_prove_many: K independent proofs of one AIR, trace length and options in one pass.  traces: a (K, width, n) array or
+        a list of K (width, n) arrays in HOST memory; pubs: (K, npub).  Returns the K proofs, each identical to prove() of its trace."""
+        traces = [np.ascontiguousarray(t, dtype=np.uint64) for t in traces]
+        pubs = np.ascontiguousarray(pubs, dtype=np.uint64)
+        if pubs.ndim == 1:
+            pubs = pubs.reshape(len(traces), -1)
+        if not traces or pubs.ndim != 2 or pubs.shape[0] != len(traces):
+            raise CsgError("one row of public inputs per trace expected")
+        if any(t.ndim != 2 or t.shape != traces[0].shape for t in traces) or traces[0].shape[0] != TRACE_WIDTH[air_id]:
+            raise CsgError(f"every trace must be ({TRACE_WIDTH[air_id]}, n)")
+        k = len(traces)
+        ptrs = (_u64p * k)(*[_p64(t) for t in traces])
+        outs, lens = (_u8p * k)(), (C.c_size_t * k)()
+        self._check(lib().csg_prove_many(self._h, air_id, k, ptrs, repr, traces[0].shape[1], _p64(pubs), pubs.shape[1], C.byref(options), outs, lens))
+        proofs = [C.string_at(outs[i], lens[i]) for i in range(k)]
+        for i in range(k):
+            lib().csg_free(outs[i])
+        return proofs
 
     def prove_columns(self, air_id: int, columns, pub: np.ndarray, options: ProofOptions, repr: int = REPR_CANONICAL) -> bytes:
         """csg_prove_columns: one separately allocated array per trace column (how a winterfell TraceTable holds them)"""

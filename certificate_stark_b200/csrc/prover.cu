@@ -29,6 +29,7 @@ void csg_destroy(csg_ctx *ctx) {
     for (auto b : ctx->stage_buf) if (b) cudaFreeHost(b);
     for (auto e : ctx->stage_ev) if (e) cudaEventDestroy(e);
     if (ctx->h2d_a) { cudaEventDestroy(ctx->h2d_a); cudaEventDestroy(ctx->h2d_b); }
+    many_delete(ctx->many);
     delete ctx;
     cudaStreamDestroy(s);
 }
@@ -75,6 +76,20 @@ int csg_prove_columns(csg_ctx *ctx, int air_id, const uint64_t *const *columns, 
         csg_ctx::check_repr(repr);
         ctx->set_air(air_id, trace_len, opt, pub, npub);
         ctx->prove_loaded(proof, proof_len, nullptr, repr, columns);
+    });
+}
+// K independent proofs of one AIR, length and options through one launch sequence (many/prove_many.cu).  The single-proof state
+// (AIR, resident and prefetched traces) is left alone; only the timings are the batch's.
+int csg_prove_many(csg_ctx *ctx, int air_id, size_t count, const uint64_t *const *traces, int repr, size_t trace_len, const uint64_t *pubs, size_t npub,
+                   const csg_options *opt, uint8_t **proofs, size_t *proof_lens) {
+    if (proofs && proof_lens)   // the caller's arrays hold count entries
+        for (size_t k = 0; k < count; k++) { proofs[k] = nullptr; proof_lens[k] = 0; }
+    return guarded(ctx, [&] {
+        if (ctx->comm && ctx->comm->world > 1) throw std::runtime_error("csg_prove_many does not run on a context attached to a group");
+        if (!ctx->many) ctx->many = many_new();
+        ctx->stage_timer.discard(); ctx->query_timer.discard();   // csg_get_timings reports the batch
+        try { many_prove(ctx->many, ctx->st, air_id, count, traces, repr, trace_len, pubs, npub, opt, proofs, proof_lens, ctx->tm); }
+        catch (const ManyArgError &e) { throw ArgError(e.what()); }
     });
 }
 // page-locked host memory for traces: the H2D copy of csg_prove / csg_prove_trace then runs at link speed under the extension

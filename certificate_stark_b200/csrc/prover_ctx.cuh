@@ -24,7 +24,9 @@
 #include "hash.cuh"
 #include "host/air_desc.hpp"
 #include "host/batch_plan.hpp"
+#include "host/proof_common.hpp"
 #include "host/transcript.hpp"
+#include "many/many.cuh"
 #include "ntt.cuh"
 #include "stages.cuh"
 #include "witness.cuh"
@@ -234,18 +236,11 @@ struct csg_ctx {
     float h2d_ms_last = 0;
     cudaEvent_t h2d_a = nullptr, h2d_b = nullptr;   // first byte .. last byte of the overlapped H2D copy, on the copy stream
     CosetTables lde_tables;                      // per-coset scale tables of the LDE domain, built once per csg_set_air
+    ManyProver *many = nullptr;                  // csg_prove_many: its own device buffers and tables, created by the first batch
 
     // ------------------------------------------------------------------------------------------ setup
     void set_air(int air_id, size_t trace_len, const csg_options *o, const uint64_t *pub, size_t npub) {
-        if (!o) throw ArgError("options missing");
-        if (o->field_extension < CSG_FIELD_EXT_NONE || o->field_extension > CSG_FIELD_EXT_CUBIC) throw ArgError("field extension must be None (1), Quadratic (2) or Cubic (3)");
-        if (o->fri_folding_factor != 4) throw ArgError("only FRI folding factor 4 is implemented");
-        if (o->hash_fn != CSG_HASH_BLAKE3_256 && o->hash_fn != CSG_HASH_SHA3_256) throw ArgError("hash function must be Blake3_256 or Sha3_256");
-        if (o->num_queries == 0 || o->num_queries > 255 || o->grinding_factor >= 32) throw ArgError("num_queries in 1..255, grinding factor below 32");
-        if (o->blowup_factor < 2 || o->blowup_factor > 32 || (o->blowup_factor & (o->blowup_factor - 1))) throw ArgError("blowup factor must be a power of two in 2..32");
-        // winterfell caps the remainder at 1024 elements; its byte length is serialised as a u16 (8192 elements would wrap to 0)
-        if (o->fri_max_remainder_size < 4 || o->fri_max_remainder_size > 1024 || (o->fri_max_remainder_size & (o->fri_max_remainder_size - 1)))
-            throw ArgError("FRI remainder size must be a power of two in 4..1024");
+        try { check_options(o); } catch (const std::invalid_argument &e) { throw ArgError(e.what()); }
         // The same AIR, length, options and sharding as the last call -- a prover proving batch after batch, where only the public
         // inputs (assertion values) differ: the root table, the periodic-column tables and the coset scale tables on the device
         // stay as they are, and so does a prefetched trace.
@@ -286,11 +281,7 @@ struct csg_ctx {
         if (!shard_plan(rank, G, b, ce, air.width, &plan)) throw ArgError("the number of ranks of a sharded proof must divide the blowup factor");
         bl = plan.num_cosets; k0 = plan.first_coset;
         if (logn > 22) throw ArgError("trace length above 2^22 is not supported");
-        {   // the FRI remainder layer is committed as rows of 4: it needs at least 2 rows
-            size_t m = lde_n;
-            while (m > o->fri_max_remainder_size) m /= 4;
-            if (m < 8) throw ArgError("FRI remainder would have fewer than 8 elements: raise fri_max_remainder_size");
-        }
+        try { check_remainder(lde_n, *o); } catch (const std::invalid_argument &e) { throw ArgError(e.what()); }
         if (air.num_constraints() > (size_t)CONS_MAX_CONSTRAINTS || air.periodic.size() > (size_t)CONS_MAX_PERIODIC ||
             air.assertions.size() > (size_t)CONS_MAX_ASSERTIONS)
             throw ArgError("AIR exceeds the compiled table sizes");
@@ -695,7 +686,7 @@ struct csg_ctx {
                 A.a_value[i] = s.values[0]; A.a_poly_len[i] = (unsigned)s.values.size(); A.a_poly_off[i] = polys.size();
                 A.a_xoff[i] = s.first_step ? f63::pow(g_inv, s.first_step) : ONE;
                 if (s.values.size() > 1) {
-                    std::vector<fe> c = host_interpolate(s.values);
+                    std::vector<fe> c = interpolate_host(s.values);
                     polys.insert(polys.end(), c.begin(), c.end());
                 }
             }
@@ -757,19 +748,6 @@ struct csg_ctx {
         for (size_t i = 0; i < 2 * na; i++) bj[i] = b_ab[i].c[0];
         eval_constraints(tj.data(), bj.data(), 0, true);
     }
-    // coefficients of the polynomial taking the given values on <w_len> (host, tiny: one value per signature)
-    static std::vector<fe> host_interpolate(const std::vector<fe> &vals) {
-        const size_t len = vals.size();
-        const fe w_inv = inv(root_of_unity(ilog2(len))), len_inv = inv(to_mont(len));
-        std::vector<fe> c(len);
-        for (size_t m = 0; m < len; m++) {
-            fe s = 0, wm = f63::pow(w_inv, m), x = ONE;
-            for (size_t i = 0; i < len; i++) { s = add(s, mul(vals[i], x)); x = mul(x, wm); }
-            c[m] = mul(s, len_inv);
-        }
-        return c;
-    }
-
     // ------------------------------------------------------------------------------------------ stage 4
     void commit_composition(uint8_t root[32]) {
         need(S_EVALUATED, "constraints must be evaluated first");
@@ -1006,7 +984,7 @@ struct csg_ctx {
         nfri++;
         t.stop(st, &tm.fri, true); tm.stage_launches[5] += t.launches;
     }
-    size_t num_fri_folds() const { size_t r = 0, d = lde_n; while (d > opt.fri_max_remainder_size) { d /= 4; r++; } return r; }
+    size_t num_fri_folds() const { return csg::num_fri_folds(lde_n, opt); }
 
     // ------------------------------------------------------------------------------------------ stage 9
     void upload_positions(const std::vector<uint32_t> &p32) {
@@ -1065,20 +1043,8 @@ struct csg_ctx {
         }
         return out;
     }
-    static std::vector<size_t> fold_positions(const std::vector<size_t> &pos, size_t domain) {
-        std::vector<size_t> out;
-        for (size_t p : pos) { size_t f = p % (domain / 4); if (std::find(out.begin(), out.end(), f) == out.end()) out.push_back(f); }
-        return out;
-    }
-
     // ------------------------------------------------------------------------------------------ the whole of Prover::prove
-    void write_context(Bytes &w) const {
-        w.u8((uint8_t)air.width); w.u8((uint8_t)logn); w.u16(0);
-        w.u8(8); w.u64(P);
-        w.u8((uint8_t)opt.num_queries); w.u8((uint8_t)ilog2(opt.blowup_factor)); w.u8((uint8_t)opt.grinding_factor);
-        w.u8((uint8_t)opt.hash_fn); w.u8((uint8_t)opt.field_extension);
-        w.u8((uint8_t)ilog2(opt.fri_folding_factor)); w.u8((uint8_t)ilog2(opt.fri_max_remainder_size));
-    }
+    void write_context(Bytes &w) const { write_proof_context(w, air.width, logn, opt); }
     // flattened components of E elements (serialisation / hashing order)
     std::vector<fe> flat(const std::vector<xe> &v) const {
         std::vector<fe> out;
@@ -1161,12 +1127,6 @@ struct csg_ctx {
         std::vector<size_t> pos = coin.draw_integers(opt.num_queries, lde_n);
         mark("grinding + positions");
 
-        Bytes pf;
-        pf.v.reserve(256 * 1024);
-        write_context(pf);
-        pf.u16((uint16_t)((2 + nlayers) * 32));
-        pf.put(trace_root, 32); pf.put(comp_root, 32);
-        for (auto &r : fri_roots) pf.put(r.data(), 32);
         // every opening of the proof -- trace rows, composition rows, FRI layer rows, their Merkle paths, the remainder -- is
         // planned on the host first and fetched in ONE round trip (one index upload, a handful of gather launches, one download)
         OpenBatch B;
@@ -1193,28 +1153,12 @@ struct csg_ctx {
         mark("plan openings");
         run_openings(B, rows, digs, last, rem_off);
         mark("openings round trip");
-        auto emit = [&](const Opening &o) {
-            pf.u32((uint32_t)(o.rows_len * 8));
-            pf.u64s(rows.data() + o.rows_off, o.rows_len);
-            Bytes paths;
-            paths.u8((uint8_t)o.slots.size());
-            size_t at = o.dig_off;
-            for (auto &sl : o.slots) { paths.u8((uint8_t)sl.size()); paths.put(digs.data() + at * 32, sl.size() * 32); at += sl.size(); }
-            pf.u32((uint32_t)paths.v.size()); pf.put(paths.v.data(), paths.v.size());
-        };
-        emit(o_trace);
-        emit(o_comp);
-        pf.u16((uint16_t)(w * d * 8));
-        for (fe v : flat(xood_cur)) pf.element(v);
-        for (fe v : flat(xood_next)) pf.element(v);
-        pf.u16((uint16_t)(ce * d * 8));
-        for (fe v : flat(xood_comp)) pf.element(v);
-        pf.u8((uint8_t)(nlayers - 1));
-        for (const Opening &o : o_fri) emit(o);
-        pf.u16((uint16_t)(rem_len * 8));
-        pf.u64s(rows.data() + rem_off, rem_len);
-        pf.u8(1);
-        pf.u64(nonce);
+        Bytes pf;
+        pf.v.reserve(256 * 1024);
+        std::vector<const uint8_t *> fri_root_ptrs;
+        for (auto &r : fri_roots) fri_root_ptrs.push_back(r.data());
+        write_proof(pf, (unsigned)w, logn, opt, trace_root, comp_root, fri_root_ptrs, o_trace, o_comp, o_fri, rows.data(), digs.data(), flat(xood_cur),
+                    flat(xood_next), flat(xood_comp), rem_off, rem_len, nonce);
         tq.stop(st, &tm.queries); tm.stage_launches[6] = tq.launches;
         mark("serialise");
         tm.kernel_launches = st.launches - launches0;
@@ -1234,7 +1178,6 @@ struct csg_ctx {
         stage = S_TRACE;   // the resident trace (d_io) can be proved again
     }
     // ---- batched openings
-    struct Opening { size_t rows_off = 0, rows_len = 0, dig_off = 0; std::vector<std::vector<uint32_t>> slots; };
     struct OpenBatch {
         struct Rows { const fe *data; unsigned width, ncosets; size_t coset_stride, col_stride; unsigned sub; size_t sub_stride, idx_off, npos, rows_off; };
         struct Digs { const uint32_t *nodes, *top; size_t idx_off, count, dig_off; };

@@ -88,6 +88,19 @@ int csg_prove(csg_ctx *ctx, int air_id, const uint64_t *trace, int repr, size_t 
 int csg_prove_columns(csg_ctx *ctx, int air_id, const uint64_t *const *columns, int repr, size_t trace_len, const uint64_t *pub, size_t npub,
                       const csg_options *opt, uint8_t **proof, size_t *proof_len);
 
+/* K independent proofs of one AIR, one trace length and one csg_options: traces[k] is a column-major [width][trace_len]
+ * trace (repr as in csg_prove), pubs = K * npub public-input words.  proofs[k] receives a malloc'ed proof that is
+ * byte-identical to what csg_prove would return for (traces[k], pubs + k*npub); release each with csg_free.  On failure
+ * every proofs[k] is NULL.
+ * Every stage runs as one launch sequence over all K proofs and every Fiat-Shamir step is one device->host copy for the batch, so
+ * launches and round trips are paid once per batch: the call is for many small proofs (range proofs, signatures, Rescue chains).
+ * The context's single-proof state (csg_set_air, the resident and the prefetched trace) is not touched; the batch keeps its own
+ * device buffers, reused by the next batch of the same shape and freed by csg_destroy.  csg_get_timings then reports the batch.
+ * CSG_ERR_UNSUPPORTED: field_extension 2 or 3, a context attached to a group (world > 1), trace_len > 2^16.
+ * CSG_ERR_ARG: count == 0 or count > 1024, count * width > 65535, null pointers, a bad repr or npub, a batch whose device
+ * footprint does not fit the free memory.  All checks run before anything is enqueued. */
+int csg_prove_many(csg_ctx *ctx, int air_id, size_t count, const uint64_t *const *traces, int repr, size_t trace_len,
+                   const uint64_t *pubs, size_t npub, const csg_options *opt, uint8_t **proofs, size_t *proof_lens);
 /* ---- verification: replaces `winterfell::verify::<Air>(proof, pub_inputs)` (src/lib.rs:144-150).  Host-only, as in the
  * reference; needs no context and no GPU.  Returns CSG_OK or one of CSG_VERIFY_*. */
 int csg_verify(int air_id, const uint64_t *pub, size_t npub, const uint8_t *proof, size_t proof_len);
