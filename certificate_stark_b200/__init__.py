@@ -85,6 +85,10 @@ def lib() -> C.CDLL:
         "csg_create": (vp, [C.c_int]), "csg_destroy": (None, [vp]), "csg_last_error": (C.c_char_p, [vp]), "csg_free": (None, [vp]),
         "csg_prove": (C.c_int, [vp, C.c_int, _u64p, C.c_int, C.c_size_t, _u64p, C.c_size_t, opt, C.POINTER(_u8p), _szp]),
         "csg_prove_many": (C.c_int, [vp, C.c_int, C.c_size_t, C.POINTER(_u64p), C.c_int, C.c_size_t, _u64p, C.c_size_t, opt, C.POINTER(_u8p), _szp]),
+        "csg_prove_many_device": (C.c_int, [vp, C.c_int, C.c_size_t, vp, C.c_int, C.c_size_t, _u64p, C.c_size_t, opt, C.POINTER(_u8p), _szp]),
+        "csg_build_traces_many_rescue": (C.c_int, [vp, _u64p, C.c_size_t, C.c_size_t, vp, _u64p]),
+        "csg_build_traces_many_schnorr": (C.c_int, [vp, vp, vp, _u64p]), "csg_build_traces_many_merkle_update": (C.c_int, [vp, vp, vp, _u64p]),
+        "csg_build_traces_many_transaction": (C.c_int, [vp, vp, vp, _u64p]),
         "csg_prove_columns": (C.c_int, [vp, C.c_int, C.POINTER(_u64p), C.c_int, C.c_size_t, _u64p, C.c_size_t, opt, C.POINTER(_u8p), _szp]),
         "csg_set_air": (C.c_int, [vp, C.c_int, C.c_size_t, opt, _u64p, C.c_size_t]),
         "csg_load_trace": (C.c_int, [vp, _u64p, C.c_int]), "csg_reload_resident_trace": (C.c_int, [vp]),
@@ -163,6 +167,7 @@ class Context:
 
     def __init__(self, device: int = 0):
         self._h = lib().csg_create(device)
+        self.device = device
         if not self._h:
             raise CsgError(f"cannot open CUDA device {device}: the CUDA backend is required, there is no CPU fallback")
 
@@ -247,6 +252,61 @@ class Context:
         for i in range(k):
             lib().csg_free(outs[i])
         return proofs
+
+    def prove_many_device(self, air_id: int, traces, pubs, options: ProofOptions, repr: int = REPR_CANONICAL) -> list:
+        """csg_prove_many_device: prove_many of K traces already in device memory.  traces: a contiguous int64 / uint64 torch CUDA
+        tensor (K, width, n) on this context's device, read in place and never written.  Torch's current stream is synchronised
+        first, so work queued on it that writes the tensor has finished."""
+        import torch
+        if not isinstance(traces, torch.Tensor) or traces.device.type != "cuda":
+            raise CsgError("traces must be a torch CUDA tensor (K, width, n)")
+        if traces.dtype not in (torch.int64, torch.uint64) or not traces.is_contiguous():
+            raise CsgError("traces must be a contiguous int64 or uint64 tensor")
+        if traces.ndim != 3 or traces.shape[1] != TRACE_WIDTH[air_id]:
+            raise CsgError(f"traces must be (K, {TRACE_WIDTH[air_id]}, n)")
+        k = traces.shape[0]
+        pubs = np.ascontiguousarray(pubs, dtype=np.uint64).reshape(k, -1)
+        torch.cuda.current_stream(traces.device).synchronize()
+        outs, lens = (_u8p * max(k, 1))(), (C.c_size_t * max(k, 1))()
+        self._check(lib().csg_prove_many_device(self._h, air_id, k, traces.data_ptr(), repr, traces.shape[2], _p64(pubs), pubs.shape[1],
+                                                C.byref(options), outs, lens))
+        proofs = [C.string_at(outs[i], lens[i]) for i in range(k)]
+        for i in range(k):
+            lib().csg_free(outs[i])
+        return proofs
+
+    def _device_traces(self, count: int, width: int, rows: int):
+        import torch
+        return torch.empty((count, width, rows), dtype=torch.uint64, device=f"cuda:{self.device}")
+
+    def build_many_rescue(self, seeds, chain_length: int):
+        """csg_build_traces_many_rescue: K Rescue chains on the device.  seeds: (K, 7) words -> (uint64 CUDA tensor (K, 14, 8 *
+        chain_length), pubs (K, 14)), each equal to build_rescue_trace(seeds[k], chain_length)"""
+        seeds = np.ascontiguousarray(seeds, dtype=np.uint64).reshape(-1, 7)
+        k = seeds.shape[0]
+        if chain_length < 1 or chain_length & (chain_length - 1) or chain_length > 8192:
+            raise CsgError("invalid argument: chain_length must be a power of two of at most 8192")
+        out, pubs = self._device_traces(k, 14, 8 * chain_length), np.zeros((k, 14), dtype=np.uint64)
+        self._check(lib().csg_build_traces_many_rescue(self._h, _p64(seeds), k, chain_length, out.data_ptr(), _p64(pubs)))
+        return out, pubs
+
+    def build_many_schnorr(self, batch: "SignatureBatch"):
+        """csg_build_traces_many_schnorr: one trace per signature on the device -> (uint64 CUDA tensor (K, 56, 512), pubs (K, 38))"""
+        out, pubs = self._device_traces(batch.num_sig, 56, 512), np.zeros((batch.num_sig, 38), dtype=np.uint64)
+        self._check(lib().csg_build_traces_many_schnorr(self._h, batch._h, out.data_ptr(), _p64(pubs)))
+        return out, pubs
+
+    def build_many_merkle_update(self, batch: "TransactionBatch"):
+        """csg_build_traces_many_merkle_update: one trace per transfer -> (uint64 CUDA tensor (K, 65, 512), pubs (K, 14))"""
+        out, pubs = self._device_traces(batch.num_tx, 65, 512), np.zeros((batch.num_tx, 14), dtype=np.uint64)
+        self._check(lib().csg_build_traces_many_merkle_update(self._h, batch._h, out.data_ptr(), _p64(pubs)))
+        return out, pubs
+
+    def build_many_transaction(self, batch: "TransactionBatch"):
+        """csg_build_traces_many_transaction: one trace per transfer -> (uint64 CUDA tensor (K, 94, 1024), pubs (K, 14))"""
+        out, pubs = self._device_traces(batch.num_tx, 94, 1024), np.zeros((batch.num_tx, 14), dtype=np.uint64)
+        self._check(lib().csg_build_traces_many_transaction(self._h, batch._h, out.data_ptr(), _p64(pubs)))
+        return out, pubs
 
     def prove_columns(self, air_id: int, columns, pub: np.ndarray, options: ProofOptions, repr: int = REPR_CANONICAL) -> bytes:
         """csg_prove_columns: one separately allocated array per trace column (how a winterfell TraceTable holds them)"""

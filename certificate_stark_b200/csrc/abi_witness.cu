@@ -1,6 +1,22 @@
 // libcsg: device-side witnesses and batch metadata, timers and the sharding entry points of include/csg.h.
 #include "prover_ctx.cuh"
 
+// the batch witness builders below: csg_get_timings then reports the build, its kernel launches and wall time
+template <class F>
+static int build_traces_many(csg_ctx *ctx, F build) {
+    return guarded(ctx, [&] {
+        if (!ctx->many) ctx->many = many_new();
+        const auto t0 = std::chrono::steady_clock::now();
+        const unsigned long long launches0 = ctx->st.launches;
+        try { build(); }
+        catch (const ManyArgError &e) { throw ArgError(e.what()); }
+        ctx->stage_timer.discard(); ctx->query_timer.discard();
+        ctx->tm = csg_timings{};
+        ctx->tm.kernel_launches = ctx->st.launches - launches0;
+        ctx->tm.total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    });
+}
+
 extern "C" {
 
 int csg_build_trace_transaction_device(csg_ctx *ctx, const csg_tx_batch *b) {
@@ -71,6 +87,20 @@ int csg_build_trace_schnorr_device(csg_ctx *ctx, const csg_sig_batch *b) {
         ctx->tm.h2d = t.stop(ctx->st);
         ctx->nfri = 0; ctx->stage = S_TRACE;
     });
+}
+// K traces of a csg_prove_many_device batch built on the device into the caller's buffer (many/witness_many.cu).  The batch's
+// scratch is its own: the single-proof state (d_wit_in, the packed batch, the resident trace) is left alone.
+int csg_build_traces_many_rescue(csg_ctx *ctx, const uint64_t *seeds, size_t count, size_t chain_length, uint64_t *traces_dev, uint64_t *pubs) {
+    return build_traces_many(ctx, [&] { many_build_rescue(ctx->many, ctx->st, seeds, count, chain_length, traces_dev, pubs); });
+}
+int csg_build_traces_many_schnorr(csg_ctx *ctx, const csg_sig_batch *b, uint64_t *traces_dev, uint64_t *pubs) {
+    return build_traces_many(ctx, [&] { many_build_items(ctx->many, ctx->st, CSG_AIR_SCHNORR, b, traces_dev, pubs); });
+}
+int csg_build_traces_many_merkle_update(csg_ctx *ctx, const csg_tx_batch *b, uint64_t *traces_dev, uint64_t *pubs) {
+    return build_traces_many(ctx, [&] { many_build_items(ctx->many, ctx->st, CSG_AIR_MERKLE_UPDATE, b, traces_dev, pubs); });
+}
+int csg_build_traces_many_transaction(csg_ctx *ctx, const csg_tx_batch *b, uint64_t *traces_dev, uint64_t *pubs) {
+    return build_traces_many(ctx, [&] { many_build_items(ctx->many, ctx->st, CSG_AIR_TRANSACTION, b, traces_dev, pubs); });
 }
 // TransactionMetadata::build_random on the device: plan on the host (draws + tree shape, no hashing), hashes on the GPU
 int csg_tx_batch_build_device(csg_ctx *ctx, uint64_t seed, size_t num_tx, unsigned tree_depth, uint64_t pub[14]) {

@@ -97,7 +97,7 @@ size_t ntt_group_tmp(size_t ncols, size_t ncosets, size_t n) {   // the pass-A s
 class ManyProver {
   public:
     ~ManyProver() { for (auto e : ev) if (e) cudaEventDestroy(e); for (auto e : ev_cargs) if (e) cudaEventDestroy(e); }
-    void prove(Stream &st, int air_id, size_t K, const uint64_t *const *traces, int repr, size_t trace_len, const uint64_t *pubs, size_t npub,
+    void prove(Stream &st, int air_id, size_t K, ManyTraces traces, int repr, size_t trace_len, const uint64_t *pubs, size_t npub,
                const csg_options *o, uint8_t **proofs, size_t *proof_lens, csg_timings &tm);
 
   private:
@@ -121,6 +121,8 @@ class ManyProver {
     PinnedBuf<uint64_t> h_io;
     PinnedBuf<ConsArgs> h_cargs;
     cudaEvent_t ev[9] = {}, ev_cargs[2] = {};   // stage boundaries; the upload of the constraint arguments (CSG_HOST_TRACE)
+    ManyWitnessScratch wit;                     // the batch witness builders' (witness_many.cu); prove does not use it
+    friend ManyWitnessScratch &many_scratch(ManyProver *m);
 
     size_t held_bytes() const {
         size_t s = d_io.n * 8 + d_out.n * 8 + (d_tnodes.n + d_cnodes.n + d_idx.n) * 4 + d_cargs.n * sizeof(ConsArgs) + d_dargs.n * sizeof(DeepArgs) +
@@ -135,13 +137,23 @@ class ManyProver {
 
 ManyProver *many_new() { return new ManyProver(); }
 void many_delete(ManyProver *m) { delete m; }
+ManyWitnessScratch &many_scratch(ManyProver *m) { return m->wit; }
 
-void many_prove(ManyProver *m, Stream &st, int air_id, size_t count, const uint64_t *const *traces, int repr, size_t trace_len, const uint64_t *pubs,
+void check_device_buffer(const void *p, const char *what) {
+    int device = 0;
+    CSG_CUDA(cudaGetDevice(&device));
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); a.type = cudaMemoryTypeUnregistered; }
+    if (a.type != cudaMemoryTypeDevice || a.device != device)
+        throw ManyArgError(std::string(what) + " must be device memory of the context's device (not host, pinned host or managed memory)");
+}
+
+void many_prove(ManyProver *m, Stream &st, int air_id, size_t count, ManyTraces traces, int repr, size_t trace_len, const uint64_t *pubs,
                 size_t npub, const csg_options *opt, uint8_t **proofs, size_t *proof_lens, csg_timings &tm) {
     m->prove(st, air_id, count, traces, repr, trace_len, pubs, npub, opt, proofs, proof_lens, tm);
 }
 
-void ManyProver::prove(Stream &st, int air_id, size_t K, const uint64_t *const *traces, int repr, size_t trace_len, const uint64_t *pubs, size_t npub,
+void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int repr, size_t trace_len, const uint64_t *pubs, size_t npub,
                        const csg_options *o, uint8_t **proofs, size_t *proof_lens, csg_timings &tm) {
     const auto t0 = std::chrono::steady_clock::now();
     static const bool host_trace = getenv("CSG_HOST_TRACE") != nullptr;
@@ -149,14 +161,15 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, const uint64_t *const *
     struct TraceScope { bool on; TraceScope(bool o_, HostTrace *t) : on(o_) { if (on) g_host_trace = t; } ~TraceScope() { if (on) g_host_trace = nullptr; } } trace_scope(host_trace, &trace);
 
     // ------------------------------------------------------------------ every check before anything is enqueued
-    if (!traces || !pubs || !proofs || !proof_lens) throw ManyArgError("null argument");
+    if ((!traces.host && !traces.dev) || !pubs || !proofs || !proof_lens) throw ManyArgError("null argument");
     if (K == 0 || K > MANY_MAX_COUNT) throw ManyArgError("count must be in 1..1024");
     for (size_t k = 0; k < K; k++) { proofs[k] = nullptr; proof_lens[k] = 0; }
     try { check_options(o); } catch (const std::invalid_argument &e) { throw ManyArgError(e.what()); }
     if (o->field_extension != CSG_FIELD_EXT_NONE) throw ManyUnsupported("csg_prove_many proves over the base field only (field_extension 1)");
     if (trace_len > ((size_t)1 << MANY_MAX_LOG_TRACE)) throw ManyUnsupported("csg_prove_many takes traces of at most 2^16 rows: prove longer ones with csg_prove");
     if (repr != CSG_REPR_CANONICAL && repr != CSG_REPR_MONTGOMERY) throw ManyArgError("repr must be CSG_REPR_CANONICAL or CSG_REPR_MONTGOMERY");
-    for (size_t k = 0; k < K; k++) if (!traces[k]) throw ManyArgError("null trace");
+    if (traces.host) { for (size_t k = 0; k < K; k++) if (!traces.host[k]) throw ManyArgError("null trace"); }
+    else check_device_buffer(traces.dev, "the traces");
     std::vector<AirDesc> airs(K);
     try { parallel_proofs(K, [&](size_t k) { airs[k] = make_air(air_id, trace_len, pubs + k * npub, npub); }); }
     catch (const std::invalid_argument &e) { throw ManyArgError(e.what()); }
@@ -198,7 +211,8 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, const uint64_t *const *
     }
     const size_t tmp = std::max({lg > 11 ? ntt_group_tmp(K * w, nb, trace_len) : 0, lg > 11 ? ntt_group_tmp(K * ce, nb, trace_len) : 0,
                                  lg > 11 ? ntt_group_tmp(3 * K, nb, trace_len) : 0, K * w * trace_len, K * ce * trace_len});
-    const size_t need = 8 * (2 * K * w * trace_len + nb * K * w * trace_len + K * ptotal * (2 + ce) + K * npoly + K * items * ce * trace_len +
+    const size_t staged = traces.host ? K * w * trace_len : 0;   // d_io: host traces go up into it, device traces are read in place
+    const size_t need = 8 * (staged + K * w * trace_len + nb * K * w * trace_len + K * ptotal * (2 + ce) + K * npoly + K * items * ce * trace_len +
                              CONS_MAX_BGROUPS * ce * trace_len + 3 * K * ce * trace_len + nb * K * ce * trace_len + 3 * K * trace_len * (1 + nb) +
                              K * lde_n + layer_elems + tmp + 2 * open_words + K * 8 * (2 * w + ce)) +
                         4 * (2 * K * 16 * lde_n + layer_nodes + open_words) + K * (sizeof(ConsArgs) + sizeof(DeepArgs));
@@ -248,10 +262,14 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, const uint64_t *const *
     // ------------------------------------------------------------------ stage 1: traces up, periodic tables, LDE
     CSG_CUDA(cudaEventRecord(ev[0], st.s));
     const size_t tw = w * n;
-    h_io.reserve(K * tw);
-    d_io.reserve(K * tw);
-    parallel_proofs(K, [&](size_t k) { memcpy(h_io.p + k * tw, traces[k], tw * sizeof(uint64_t)); });
-    CSG_CUDA(cudaMemcpyAsync(d_io.p, h_io.p, K * tw * sizeof(uint64_t), cudaMemcpyHostToDevice, st.s));
+    const uint64_t *src = traces.dev;
+    if (traces.host) {
+        h_io.reserve(K * tw);
+        d_io.reserve(K * tw);
+        parallel_proofs(K, [&](size_t k) { memcpy(h_io.p + k * tw, traces.host[k], tw * sizeof(uint64_t)); });
+        CSG_CUDA(cudaMemcpyAsync(d_io.p, h_io.p, K * tw * sizeof(uint64_t), cudaMemcpyHostToDevice, st.s));
+        src = d_io.p;
+    }
     CSG_CUDA(cudaEventRecord(ev[1], st.s));
     host_mark("traces up");
     if (ptotal) {
@@ -272,8 +290,9 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, const uint64_t *const *
         }
     } else d_ptab.reserve(1);
     d_polys.reserve(K * tw); d_lde.reserve(b * K * tw);
-    // the representation change rides on the 1/n scaling of the interpolation (as in csg_ctx::extend_and_commit_trace)
-    intt_columns(roots, ntt, d_io.p, n, d_polys.p, n, K * w, logn, st, repr == CSG_REPR_MONTGOMERY ? 0 : R2, true);
+    // the representation change rides on the 1/n scaling of the interpolation (as in csg_ctx::extend_and_commit_trace); intt_columns
+    // writes only its output and its scratch, so a caller's device buffer is read in place
+    intt_columns(roots, ntt, src, n, d_polys.p, n, K * w, logn, st, repr == CSG_REPR_MONTGOMERY ? 0 : R2, true);
     coset_ntt_columns(roots, ntt, d_polys.p, n, d_lde.p, n, K * tw, K * w, logn, lde_tables, st);
     CSG_CUDA(cudaEventRecord(ev[2], st.s));
     stage_launches(0);

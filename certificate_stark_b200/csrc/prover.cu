@@ -80,8 +80,8 @@ int csg_prove_columns(csg_ctx *ctx, int air_id, const uint64_t *const *columns, 
 }
 // K independent proofs of one AIR, length and options through one launch sequence (many/prove_many.cu).  The single-proof state
 // (AIR, resident and prefetched traces) is left alone; only the timings are the batch's.
-int csg_prove_many(csg_ctx *ctx, int air_id, size_t count, const uint64_t *const *traces, int repr, size_t trace_len, const uint64_t *pubs, size_t npub,
-                   const csg_options *opt, uint8_t **proofs, size_t *proof_lens) {
+static int prove_many(csg_ctx *ctx, int air_id, size_t count, ManyTraces traces, int repr, size_t trace_len, const uint64_t *pubs, size_t npub,
+                      const csg_options *opt, uint8_t **proofs, size_t *proof_lens) {
     if (proofs && proof_lens)   // the caller's arrays hold count entries
         for (size_t k = 0; k < count; k++) { proofs[k] = nullptr; proof_lens[k] = 0; }
     return guarded(ctx, [&] {
@@ -91,6 +91,15 @@ int csg_prove_many(csg_ctx *ctx, int air_id, size_t count, const uint64_t *const
         try { many_prove(ctx->many, ctx->st, air_id, count, traces, repr, trace_len, pubs, npub, opt, proofs, proof_lens, ctx->tm); }
         catch (const ManyArgError &e) { throw ArgError(e.what()); }
     });
+}
+int csg_prove_many(csg_ctx *ctx, int air_id, size_t count, const uint64_t *const *traces, int repr, size_t trace_len, const uint64_t *pubs, size_t npub,
+                   const csg_options *opt, uint8_t **proofs, size_t *proof_lens) {
+    return prove_many(ctx, air_id, count, ManyTraces{traces, nullptr}, repr, trace_len, pubs, npub, opt, proofs, proof_lens);
+}
+// the same with the K traces in one device buffer [count][width][trace_len] on the context's device, read in place
+int csg_prove_many_device(csg_ctx *ctx, int air_id, size_t count, const uint64_t *traces_dev, int repr, size_t trace_len, const uint64_t *pubs,
+                          size_t npub, const csg_options *opt, uint8_t **proofs, size_t *proof_lens) {
+    return prove_many(ctx, air_id, count, ManyTraces{nullptr, traces_dev}, repr, trace_len, pubs, npub, opt, proofs, proof_lens);
 }
 // page-locked host memory for traces: the H2D copy of csg_prove / csg_prove_trace then runs at link speed under the extension
 void *csg_host_alloc(size_t bytes) {

@@ -14,7 +14,8 @@
  *                             keeping the transcript (RandomCoin) and proof serialisation on the Rust side.
  * plus the witness builders (build_trace of each prover) and a few kernel-level entry points used by the
  * parity tests and the kernel sweep.  All functions return 0 on success; they never unwind.  A context is
- * single-threaded and owns all device memory; every pointer argument is a HOST pointer owned by the caller.
+ * single-threaded and owns all device memory; every pointer argument is a HOST pointer owned by the caller, except the
+ * traces_dev buffers of csg_prove_many_device and csg_build_traces_many_*, which are device memory the caller owns.
  */
 #ifndef CSG_H
 #define CSG_H
@@ -101,6 +102,13 @@ int csg_prove_columns(csg_ctx *ctx, int air_id, const uint64_t *const *columns, 
  * footprint does not fit the free memory.  All checks run before anything is enqueued. */
 int csg_prove_many(csg_ctx *ctx, int air_id, size_t count, const uint64_t *const *traces, int repr, size_t trace_len,
                    const uint64_t *pubs, size_t npub, const csg_options *opt, uint8_t **proofs, size_t *proof_lens);
+/* csg_prove_many with the K traces already in device memory: traces_dev is ONE contiguous buffer [count][width][trace_len] on the
+ * context's device (cudaMalloc'ed, a torch CUDA tensor, the output of csg_build_traces_many_*).  Same checks, limits, errors and
+ * proof bytes as csg_prove_many; host, pinned host and managed memory and memory of another device are CSG_ERR_ARG.  The library
+ * reads the buffer in place and never writes it.  The caller's writes to it must have finished before the call (synchronise the
+ * stream that wrote it): the batch runs on the context's own stream. */
+int csg_prove_many_device(csg_ctx *ctx, int air_id, size_t count, const uint64_t *traces_dev, int repr, size_t trace_len,
+                          const uint64_t *pubs, size_t npub, const csg_options *opt, uint8_t **proofs, size_t *proof_lens);
 /* ---- verification: replaces `winterfell::verify::<Air>(proof, pub_inputs)` (src/lib.rs:144-150).  Host-only, as in the
  * reference; needs no context and no GPU.  Returns CSG_OK or one of CSG_VERIFY_*. */
 int csg_verify(int air_id, const uint64_t *pub, size_t npub, const uint8_t *proof, size_t proof_len);
@@ -237,6 +245,22 @@ size_t csg_sig_batch_size(const csg_sig_batch *b);
 int csg_build_trace_schnorr(const csg_sig_batch *b, uint64_t *trace /* 56 x 512*num_sig */, uint64_t *pub /* 38*num_sig */); /* src/schnorr/prover.rs:52-80 */
 int csg_build_trace_range(uint64_t number, uint64_t *trace /* 2 x 64 */, uint64_t pub[1]);                          /* src/range/prover.rs:36-56 */
 int csg_build_trace_rescue(const uint64_t seed[7], size_t chain_length, uint64_t *trace /* 14 x 8*len */, uint64_t pub[14]); /* benches/rescue.rs:279-321 */
+/* Batch witness builders for csg_prove_many_device: build the traces of count proofs ON THE DEVICE into traces_dev, a device buffer
+ * of the context's device that the caller owns and sizes [count][width][rows] (canonical words), and write the public inputs of
+ * every proof to the host array pubs in csg_prove's word order.  The device has finished when they return.  count is 1..1024;
+ * null pointers and a traces_dev that is not device memory of the context's device are CSG_ERR_ARG, checked before anything runs.
+ * The builders keep their scratch with the batch (freed by csg_destroy) and leave the single-proof state alone.
+ *   rescue:         count chains, seeds = count * 7 words (reduced mod p), rows = 8 * chain_length; chain_length a power of two
+ *                   up to 8192; trace k and pubs + 14k equal csg_build_trace_rescue(seeds + 7k, chain_length)
+ *   schnorr:        one proof per signature of the batch (56 x 512), pubs: 38 words per signature
+ *   merkle_update:  one proof per transfer (65 x 512), pubs: 14 words per transfer (root before it, root after it)
+ *   transaction:    one proof per transfer (94 x 1024), pubs as merkle_update; the batch's tree depth must be 15
+ * Trace k of the last three is columns [k * rows, (k + 1) * rows) of the host builder's trace of the whole batch (for the
+ * Merkle update with row 1 of columns 14 and 43 set to 1, as MerkleProver::build_trace sets them in every single proof). */
+int csg_build_traces_many_rescue(csg_ctx *ctx, const uint64_t *seeds, size_t count, size_t chain_length, uint64_t *traces_dev, uint64_t *pubs);
+int csg_build_traces_many_schnorr(csg_ctx *ctx, const csg_sig_batch *b, uint64_t *traces_dev, uint64_t *pubs);
+int csg_build_traces_many_merkle_update(csg_ctx *ctx, const csg_tx_batch *b, uint64_t *traces_dev, uint64_t *pubs);
+int csg_build_traces_many_transaction(csg_ctx *ctx, const csg_tx_batch *b, uint64_t *traces_dev, uint64_t *pubs);
 
 /* ---- kernel-level entry points (parity tests, kernel sweep).  Host buffers in/out; values canonical ------------- */
 /* per-column inverse NTT + coset LDE: cols [width][n] -> lde [width][n*blowup], natural order x_j = 3 * w^j */
