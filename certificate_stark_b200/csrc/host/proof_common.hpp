@@ -1,5 +1,5 @@
-// Host helpers shared by the single-proof driver (prover_ctx.cuh) and the batch driver (many/prove_many.cu): the checks on
-// ProofOptions, the serialised proof context, the interpolant of an assertion sequence and the folding of query positions.
+// Host helpers shared by the single-proof driver (prover_ctx.cuh), the batch driver (many/prove_many.cu) and the verifier: the checks
+// on ProofOptions, the serialised proof context, the interpolant of an assertion sequence and the folding of query positions.
 #pragma once
 #include <algorithm>
 #include <stdexcept>
@@ -66,6 +66,13 @@ inline std::vector<size_t> fold_positions(const std::vector<size_t> &pos, size_t
 // node indices of its BatchMerkleProof grouped the way serialize_nodes() writes them (batch_opening_nodes)
 struct Opening { size_t rows_off = 0, rows_len = 0, dig_off = 0; std::vector<std::vector<uint32_t>> slots; };
 
+// BatchMerkleProof::serialize_nodes() of an opening whose path digests sit at digs[32 * o.dig_off ..)
+inline void write_paths(Bytes &out, const Opening &o, const uint8_t *digs) {
+    out.u8((uint8_t)o.slots.size());
+    size_t at = o.dig_off;
+    for (auto &sl : o.slots) { out.u8((uint8_t)sl.size()); out.put(digs + at * 32, sl.size() * 32); at += sl.size(); }
+}
+
 // StarkProof::to_bytes: context, commitments, trace and constraint queries, out-of-domain frame, FRI layers and remainder,
 // proof-of-work nonce.  rows / digs: the opened words and the 32-byte path digests the openings index into; the frame vectors hold
 // the components of their elements in order (d per element with a field extension); the remainder is rows[rem_off, + rem_len).
@@ -77,9 +84,7 @@ inline void write_proof(Bytes &pf, unsigned width, unsigned logn, const csg_opti
         pf.u32((uint32_t)(o.rows_len * 8));
         pf.u64s(rows + o.rows_off, o.rows_len);
         Bytes paths;
-        paths.u8((uint8_t)o.slots.size());
-        size_t at = o.dig_off;
-        for (auto &sl : o.slots) { paths.u8((uint8_t)sl.size()); paths.put(digs + at * 32, sl.size() * 32); at += sl.size(); }
+        write_paths(paths, o, digs);
         pf.u32((uint32_t)paths.v.size()); pf.put(paths.v.data(), paths.v.size());
     };
     write_proof_context(pf, width, logn, opt);

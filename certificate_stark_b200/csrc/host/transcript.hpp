@@ -39,11 +39,6 @@ class Coin {
         counter_ = 0;
     }
     void reseed_with_int(uint64_t v) { uint8_t t[32]; merge_with_int(v, t); memcpy(seed_, t, 32); counter_ = 0; }
-    // rejection-samples the first 8 bytes of successive outputs until they form a canonical element
-    fe draw() {
-        for (int i = 0; i < 1000; i++) { uint64_t v = next_u64(); if (v < f63::P) return f63::to_mont(v); }
-        throw std::runtime_error("random coin failed to draw a field element");
-    }
     // an element of the degree-d extension: the first 8*d bytes of one output as d canonical words, the whole output
     // rejected unless every word is below p (coin.draw::<E>())
     // For d = 3 only 1.7 % of the outputs pass (each word is below p with probability 0.26), about 60 hashes per draw and
@@ -112,6 +107,69 @@ inline void hash_elements_host(int hash_fn, const fe *e, size_t n, uint8_t out[3
     for (size_t i = 0; i < n; i++) { uint64_t v = f63::from_mont(e[i]); memcpy(b.data() + 8 * i, &v, 8); }
     hashes::hash_bytes(hash_fn, b.data(), b.size(), out);
 }
+
+// The Fiat-Shamir schedule of Prover::prove, one method per step in protocol order.  Both provers and the verifier draw every
+// challenge through it: a proof is only valid if all three replay the same schedule.  Challenges are elements of the degree-d
+// extension (d = 1: the base field, in component 0).
+class ProofTranscript {
+  public:
+    // seeded with the public inputs as little-endian words, then the serialised proof context (write_proof_context)
+    ProofTranscript(int hash_fn, int d, const uint64_t *pub, size_t npub, const uint8_t *context, size_t context_len)
+        : hash_fn_(hash_fn), d_(d), coin_(seeded(hash_fn, pub, npub, context, context_len)) {}
+
+    // (alpha, beta) per transition constraint, then per assertion
+    struct ConstraintCoefficients { std::vector<f63::xe> transition, boundary; };
+    ConstraintCoefficients constraint_coefficients(const uint8_t trace_root[32], size_t nconstraints, size_t nassertions) {
+        coin_.reseed(trace_root);
+        std::vector<f63::xe> t = draw(2 * nconstraints);
+        return {std::move(t), draw(2 * nassertions)};
+    }
+    // the out-of-domain point z
+    f63::xe ood_point(const uint8_t comp_root[32]) { coin_.reseed(comp_root); return draw(); }
+    // (alpha, beta) per trace column, one coefficient per composition column, lambda and mu.  The frame is given as flat component
+    // arrays: cur and next hold w elements, comp ce elements, d components each.
+    struct DeepCoefficients { std::vector<f63::xe> trace, comp; f63::xe lambda, mu; };
+    DeepCoefficients deep_coefficients(const fe *cur, const fe *next, size_t w, const fe *comp, size_t ce) {
+        uint8_t dg[32];
+        hash_elements_host(hash_fn_, cur, w * d_, dg); coin_.reseed(dg);
+        hash_elements_host(hash_fn_, next, w * d_, dg); coin_.reseed(dg);
+        hash_elements_host(hash_fn_, comp, ce * d_, dg); coin_.reseed(dg);
+        DeepCoefficients c;
+        c.trace.resize(2 * w);
+        for (size_t i = 0; i < w; i++) { c.trace[2 * i] = draw(); c.trace[2 * i + 1] = draw(); (void)draw(); }   // a third per column, unused
+        c.comp = draw(ce);
+        c.lambda = draw(); c.mu = draw();
+        return c;
+    }
+    // the folding challenge of a FRI layer (also drawn for the remainder layer, which is not folded)
+    f63::xe fri_alpha(const uint8_t layer_root[32]) { coin_.reseed(layer_root); return draw(); }
+    // proof of work: the first nonce from 1 that reaches `bits` zeros (Coin::check_leading_zeros); the coin is reseeded with it
+    uint64_t grind(unsigned bits) {
+        uint64_t nonce = 1;
+        while (coin_.check_leading_zeros(nonce) < bits) nonce++;
+        coin_.reseed_with_int(nonce);
+        return nonce;
+    }
+    // the verifier's side of grind(): reseeds with the proof's nonce and checks its work
+    bool accept_nonce(uint64_t nonce, unsigned bits) { coin_.reseed_with_int(nonce); return coin_.leading_zeros() >= bits; }
+    std::vector<size_t> query_positions(size_t count, size_t domain_size) { return coin_.draw_integers(count, domain_size); }
+
+  private:
+    int hash_fn_, d_;
+    Coin coin_;
+    static Coin seeded(int hash_fn, const uint64_t *pub, size_t npub, const uint8_t *context, size_t context_len) {
+        Bytes seed;
+        seed.u64s(pub, npub);
+        seed.put(context, context_len);
+        return Coin(hash_fn, seed.v.data(), seed.v.size());
+    }
+    f63::xe draw() { return coin_.draw_x(d_); }
+    std::vector<f63::xe> draw(size_t count) {
+        std::vector<f63::xe> v(count);
+        for (f63::xe &e : v) e = draw();
+        return v;
+    }
+};
 
 // Which tree nodes a batch opening of `positions` carries, grouped the way BatchMerkleProof stores them: one vector
 // per pair of adjacent leaves touched, siblings appended level by level.  Node numbering: root 1, leaves at nleaves+j.

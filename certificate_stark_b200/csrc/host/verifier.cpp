@@ -11,6 +11,7 @@
 #include "../../../include/csg.h"
 #include "../airs.cuh"
 #include "air_desc.hpp"
+#include "proof_common.hpp"
 #include "transcript.hpp"
 
 namespace csg {
@@ -144,16 +145,17 @@ xe fold_row(int d, const xe v[4], fe x_inv, const xe &alpha, fe zeta_inv, fe qua
     for (int j = 2; j >= 0; j--) r = x_add(x_mul(d, r, y), c[j]);
     return x_scale(r, quarter);
 }
-std::vector<size_t> fold_positions(const std::vector<size_t> &pos, size_t domain) {
-    std::vector<size_t> out;
-    for (size_t p : pos) { size_t f = p % (domain / 4); if (std::find(out.begin(), out.end(), f) == out.end()) out.push_back(f); }
-    return out;
-}
 xe horner_bx(int d, const std::vector<fe> &c, const xe &x) { xe r = x_zero(); for (size_t i = c.size(); i-- > 0;) r = x_add_base(x_mul(d, r, x), c[i]); return r; }
 bool read_x(Reader &R, int d, xe &out) { out = x_zero(); for (int j = 0; j < d; j++) if (!R.element(out.c[j])) return false; return true; }
-void hash_x(int hf, int d, const xe *e, size_t n, uint8_t out[32]) {
+// the components of E elements in order (hashing and serialisation order)
+std::vector<fe> flat(int d, const xe *e, size_t n) {
     std::vector<fe> f;
     for (size_t i = 0; i < n; i++) for (int j = 0; j < d; j++) f.push_back(e[i].c[j]);
+    return f;
+}
+std::vector<fe> flat(int d, const std::vector<xe> &v) { return flat(d, v.data(), v.size()); }
+void hash_x(int hf, int d, const xe *e, size_t n, uint8_t out[32]) {
+    const std::vector<fe> f = flat(d, e, n);
     hash_elements_host(hf, f.data(), f.size(), out);
 }
 
@@ -209,7 +211,7 @@ int verify_impl(int air_id, const uint64_t *pub, size_t npub, const uint8_t *pro
     o.grinding_factor = (uint32_t)R.uint(1);
     o.hash_fn = (uint32_t)R.uint(1); o.field_extension = (uint32_t)R.uint(1);
     const size_t log_folding = R.uint(1), log_remainder = R.uint(1);
-    const size_t context_len = R.off;     // the exact context bytes seed the coin below
+    const size_t context_len = R.off;     // the exact context bytes seed the transcript below
     // the same ranges the prover enforces (prover.cu set_air): blowup 2..32, folding 4, remainder 4..1024, grinding below 32;
     // checked on the log2 bytes BEFORE shifting (a byte >= 32 would be undefined behaviour / wrap to a small value)
     if (R.bad || modlen != 8 || logn < 3 || logn > 40 || log_blowup < 1 || log_blowup > 5 || log_folding != 2 || log_remainder < 2 || log_remainder > 10 ||
@@ -235,10 +237,8 @@ int verify_impl(int air_id, const uint64_t *pub, size_t npub, const uint8_t *pro
     if (air.width != w) return CSG_VERIFY_MALFORMED;
     const size_t ce = air.ce_blowup(), nc = air.num_constraints(), na = air.assertions.size();
     if (ce > b) return CSG_VERIFY_MALFORMED;
-    size_t nfolds = 0, final_domain = lde_n;
-    for (; final_domain > o.fri_max_remainder_size; final_domain /= 4) nfolds++;
-    if (final_domain < 8) return CSG_VERIFY_MALFORMED;   // the remainder is committed as rows of 4: the prover refuses fewer than 2 rows
-    const size_t nlayers = nfolds + 1;
+    try { check_remainder(lde_n, o); } catch (const std::invalid_argument &) { return CSG_VERIFY_MALFORMED; }
+    const size_t nfolds = num_fri_folds(lde_n, o), nlayers = nfolds + 1;
 
     const size_t clen = R.uint(2); const uint8_t *commits = R.take(clen);
     if (R.bad || clen != (2 + nlayers) * 32) return CSG_VERIFY_MALFORMED;
@@ -259,18 +259,11 @@ int verify_impl(int air_id, const uint64_t *pub, size_t npub, const uint8_t *pro
     const size_t nparts = R.uint(1); const uint64_t nonce = R.uint(8);
     if (R.bad || R.off != R.len || nparts != 1) return CSG_VERIFY_MALFORMED;
 
-    // transcript
-    Bytes seed;
-    for (size_t i = 0; i < npub; i++) seed.u64(pub[i]);
-    seed.put(proof, context_len);
     try {
-        Coin coin(hf, seed.v.data(), seed.v.size());
-        coin.reseed(commits);
-        std::vector<xe> alpha(nc), beta(nc), b_alpha(na), b_beta(na);
-        for (size_t i = 0; i < nc; i++) { alpha[i] = coin.draw_x(d); beta[i] = coin.draw_x(d); }
-        for (size_t i = 0; i < na; i++) { b_alpha[i] = coin.draw_x(d); b_beta[i] = coin.draw_x(d); }
-        coin.reseed(commits + 32);
-        const xe z = coin.draw_x(d);
+        // the transcript, seeded with the exact context bytes of the proof
+        ProofTranscript tr(hf, d, pub, npub, proof, context_len);
+        const ProofTranscript::ConstraintCoefficients cc = tr.constraint_coefficients(commits, nc, na);
+        const xe z = tr.ood_point(commits + 32);
 
         // out-of-domain consistency: merged constraints at z against the composition columns at z^ce
         const TransitionGroups tg = transition_groups(air);
@@ -291,13 +284,12 @@ int verify_impl(int air_id, const uint64_t *pub, size_t npub, const uint8_t *pro
                 for (auto &v : ood_cur) c1.push_back(v.c[0]);
                 for (auto &v : ood_next) n1.push_back(v.c[0]);
                 for (auto &v : pv) p1.push_back(v.c[0]);
-                for (auto &v : alpha) a1.push_back(v.c[0]);
-                for (auto &v : beta) b1.push_back(v.c[0]);
+                for (size_t i = 0; i < nc; i++) { a1.push_back(cc.transition[2 * i].c[0]); b1.push_back(cc.transition[2 * i + 1].c[0]); }
                 for (auto &v : xp) x1.push_back(v.c[0]);
                 t = x_from(eval_merged_any(air_id, air, tg, c1, n1, p1, a1, b1, x1));
             } else {
                 std::vector<xe> coef(nc);
-                for (size_t i = 0; i < nc; i++) coef[i] = x_add(alpha[i], x_mul(d, beta[i], xp[tg.group_of[i]]));
+                for (size_t i = 0; i < nc; i++) coef[i] = x_add(cc.transition[2 * i], x_mul(d, cc.transition[2 * i + 1], xp[tg.group_of[i]]));
                 if (!merged_at_ext_frame(air_id, air, tg, d, ood_cur, ood_next, pv, coef, t)) return CSG_VERIFY_MALFORMED;
             }
             xe lhs = x_mul(d, x_mul(d, t, x_sub(z, x_from(f63::pow(g, n - 1)))), x_inv(d, x_sub(x_pow(d, z, n), x_one()), xk));
@@ -315,7 +307,7 @@ int verify_impl(int air_id, const uint64_t *pub, size_t npub, const uint8_t *pro
                         host_ntt(poly, true);
                         v = horner_bx(d, poly, s.first_step ? x_scale(z, f63::pow(g_inv, s.first_step)) : z);
                     }
-                    acc = x_add(acc, x_mul(d, x_sub(ood_cur[s.column], v), x_add(b_alpha[a], x_mul(d, b_beta[a], xpb))));
+                    acc = x_add(acc, x_mul(d, x_sub(ood_cur[s.column], v), x_add(cc.boundary[2 * a], x_mul(d, cc.boundary[2 * a + 1], xpb))));
                 }
                 lhs = x_add(lhs, x_mul(d, acc, x_inv(d, x_sub(x_pow(d, z, G.num_steps), x_from(G.offset)), xk)));
             }
@@ -323,19 +315,11 @@ int verify_impl(int air_id, const uint64_t *pub, size_t npub, const uint8_t *pro
             for (size_t r = 0; r < ce; r++) { rhs = x_add(rhs, x_mul(d, zp, ood_comp[r])); zp = x_mul(d, zp, z); }
             if (!x_eq(lhs, rhs)) return CSG_VERIFY_OOD_MISMATCH;
         }
-        uint8_t dg[32];
-        hash_x(hf, d, ood_cur.data(), w, dg); coin.reseed(dg);
-        hash_x(hf, d, ood_next.data(), w, dg); coin.reseed(dg);
-        hash_x(hf, d, ood_comp.data(), ce, dg); coin.reseed(dg);
-        std::vector<xe> da(w), db(w), dc(ce);
-        for (size_t c = 0; c < w; c++) { da[c] = coin.draw_x(d); db[c] = coin.draw_x(d); (void)coin.draw_x(d); }
-        for (size_t r = 0; r < ce; r++) dc[r] = coin.draw_x(d);
-        const xe lambda = coin.draw_x(d), mu = coin.draw_x(d);
+        const ProofTranscript::DeepCoefficients dc = tr.deep_coefficients(flat(d, ood_cur).data(), flat(d, ood_next).data(), w, flat(d, ood_comp).data(), ce);
         std::vector<xe> alphas(nlayers);
-        for (size_t l = 0; l < nlayers; l++) { coin.reseed(commits + (2 + l) * 32); alphas[l] = coin.draw_x(d); }
-        coin.reseed_with_int(nonce);
-        if (coin.leading_zeros() < o.grinding_factor) return CSG_VERIFY_POW;
-        const std::vector<size_t> pos = coin.draw_integers(nq, lde_n);
+        for (size_t l = 0; l < nlayers; l++) alphas[l] = tr.fri_alpha(commits + (2 + l) * 32);
+        if (!tr.accept_nonce(nonce, o.grinding_factor)) return CSG_VERIFY_POW;
+        const std::vector<size_t> pos = tr.query_positions(nq, lde_n);
 
         // openings against both commitments
         std::vector<fe> t_rows(nq * w);
@@ -360,12 +344,12 @@ int verify_impl(int air_id, const uint64_t *pub, size_t npub, const uint8_t *pro
                 xe a = x_zero(), bsum = x_zero(), csum = x_zero();
                 for (size_t c = 0; c < w; c++) {
                     const xe tv1 = x_from(t_rows[i * w + c]);
-                    a = x_add(a, x_mul(d, da[c], x_sub(tv1, ood_cur[c])));
-                    bsum = x_add(bsum, x_mul(d, db[c], x_sub(tv1, ood_next[c])));
+                    a = x_add(a, x_mul(d, dc.trace[2 * c], x_sub(tv1, ood_cur[c])));
+                    bsum = x_add(bsum, x_mul(d, dc.trace[2 * c + 1], x_sub(tv1, ood_next[c])));
                 }
-                for (size_t r = 0; r < ce; r++) csum = x_add(csum, x_mul(d, dc[r], x_sub(c_rows[i * ce + r], ood_comp[r])));
+                for (size_t r = 0; r < ce; r++) csum = x_add(csum, x_mul(d, dc.comp[r], x_sub(c_rows[i * ce + r], ood_comp[r])));
                 const xe s = x_add(x_add(x_mul(d, a, x_inv(d, x_sub(x, z), xk)), x_mul(d, bsum, x_inv(d, x_sub(x, zg), xk))), x_mul(d, csum, x_inv(d, x_sub(x, zm), xk)));
-                evals[i] = x_mul(d, s, x_add(lambda, x_scale(mu, xb)));
+                evals[i] = x_mul(d, s, x_add(dc.lambda, x_scale(dc.mu, xb)));
             }
         }
         // FRI

@@ -1,7 +1,7 @@
 // The batch driver of csg_prove_many (many.cuh): Prover::prove for K independent traces of one AIR, one length and one set of
 // options, stage by stage as csg_ctx::prove_loaded runs it, with every stage one launch sequence over all K proofs
 // (many_kernels.cuh) and every step of the Fiat-Shamir transcript one device->host copy for the whole batch.  The K transcripts run
-// on the host, one Coin per proof, spread over the host threads; a proof's transcript depends on nothing but its own trace and
+// on the host, one ProofTranscript per proof, spread over the host threads; a proof's transcript depends on nothing but its own trace and
 // public inputs, so the bytes do not depend on the thread count.
 //
 // Unlike the single-proof driver this one has no low-degree split, no sharding, no extension fields, no chunked or prefetched
@@ -19,6 +19,7 @@
 #include "../constraints.cuh"
 #include "../host/air_desc.hpp"
 #include "../host/proof_common.hpp"
+#include "../host/stage_args.hpp"
 #include "../host/transcript.hpp"
 #include "../ntt.cuh"
 #include "../stages.cuh"
@@ -68,7 +69,7 @@ void parallel_proofs(size_t count, F f) {
 
 // what one proof of the batch carries through the stages
 struct ProofState {
-    Coin coin;
+    ProofTranscript tr;
     uint8_t trace_root[32], comp_root[32];
     std::vector<std::array<uint8_t, 32>> fri_roots;
     fe z = 0;
@@ -83,7 +84,7 @@ struct ProofState {
     std::vector<Opening> o_fri;
     size_t rows_words = 0, dig_count = 0, rem_off = 0, rem_len = 0;
     size_t idx_base = 0, rows_base = 0, dig_base = 0;
-    explicit ProofState(Coin c) : coin(std::move(c)) {}
+    explicit ProofState(ProofTranscript t) : tr(std::move(t)) {}
 };
 
 size_t ntt_group_tmp(size_t ncols, size_t ncosets, size_t n) {   // the pass-A scratch of coset_ntt_columns (ntt.cu)
@@ -156,9 +157,7 @@ void many_prove(ManyProver *m, Stream &st, int air_id, size_t count, ManyTraces 
 void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int repr, size_t trace_len, const uint64_t *pubs, size_t npub,
                        const csg_options *o, uint8_t **proofs, size_t *proof_lens, csg_timings &tm) {
     const auto t0 = std::chrono::steady_clock::now();
-    static const bool host_trace = getenv("CSG_HOST_TRACE") != nullptr;
-    HostTrace trace{t0, {}};
-    struct TraceScope { bool on; TraceScope(bool o_, HostTrace *t) : on(o_) { if (on) g_host_trace = t; } ~TraceScope() { if (on) g_host_trace = nullptr; } } trace_scope(host_trace, &trace);
+    HostTraceScope trace(t0);
 
     // ------------------------------------------------------------------ every check before anything is enqueued
     if ((!traces.host && !traces.dev) || !pubs || !proofs || !proof_lens) throw ManyArgError("null argument");
@@ -176,29 +175,13 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
     const AirDesc &air = airs[0];
     const size_t w = air.width, nb = o->blowup_factor, ce = air.ce_blowup(), lde_n = trace_len * nb, nc = air.num_constraints(), na = air.assertions.size();
     if (K * w > MANY_MAX_COLUMNS) throw ManyArgError("count * trace width must not exceed 65535");
-    if (ce > nb) throw ManyArgError("blowup factor is smaller than the constraint evaluation blowup of this AIR");
-    try { check_remainder(lde_n, *o); } catch (const std::invalid_argument &e) { throw ManyArgError(e.what()); }
-    if (nc > (size_t)CONS_MAX_CONSTRAINTS || air.periodic.size() > (size_t)CONS_MAX_PERIODIC || na > (size_t)CONS_MAX_ASSERTIONS)
-        throw ManyArgError("AIR exceeds the compiled table sizes");
     const TransitionGroups tg = transition_groups(air);
     const BoundaryGroups bg = boundary_groups(air);
-    if (tg.adj.size() > (size_t)CONS_MAX_GROUPS || bg.groups.size() > (size_t)CONS_MAX_BGROUPS) throw ManyArgError("too many constraint groups");
+    try { check_air_shape(air, tg, bg, trace_len, *o); } catch (const std::invalid_argument &e) { throw ManyArgError(e.what()); }
     const unsigned lg = ilog2(trace_len);
     const size_t nfold = num_fri_folds(lde_n, *o), nlayers = nfold + 1, nq = o->num_queries;
-    // periodic columns: runs of equal period go through the transforms together; proof k's copy of column c of run [c0, c1) of period
-    // P sits at K * off(c0) + (k * (c1 - c0) + c - c0) * P of each ce coset's block of K * total elements
-    struct Run { size_t c0, c1, P, off; };
-    std::vector<Run> runs;
-    size_t ptotal = 0;
-    for (size_t c = 0; c < air.periodic.size();) {
-        const size_t P = air.periodic[c].values.size();
-        if (P == 0 || (P & (P - 1)) || P > trace_len) throw ManyArgError("periodic column length must be a power of two dividing the trace length");
-        size_t c1 = c;
-        while (c1 < air.periodic.size() && air.periodic[c1].values.size() == P) c1++;
-        runs.push_back({c, c1, P, ptotal});
-        ptotal += (c1 - c) * P;
-        c = c1;
-    }
+    const PeriodicRuns pr = periodic_runs(air);
+    const size_t ptotal = pr.total;
     size_t npoly = 0;   // coefficients of the assertion sequences of one proof
     for (const Assertion &s : air.assertions) if (s.values.size() > 1) npoly += s.values.size();
     const size_t items = constraint_items_many(air_id);
@@ -252,12 +235,9 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
 
     std::vector<ProofState> ps;
     ps.reserve(K);
-    for (size_t k = 0; k < K; k++) {
-        Bytes seed;
-        for (uint64_t v : airs[k].pub_inputs) seed.u64(v);
-        write_proof_context(seed, (unsigned)w, lg, *o);
-        ps.emplace_back(Coin(hf, seed.v.data(), seed.v.size()));
-    }
+    Bytes context;
+    write_proof_context(context, (unsigned)w, lg, *o);
+    for (size_t k = 0; k < K; k++) ps.emplace_back(ProofTranscript(hf, 1, airs[k].pub_inputs.data(), airs[k].pub_inputs.size(), context.v.data(), context.v.size()));
 
     // ------------------------------------------------------------------ stage 1: traces up, periodic tables, LDE
     CSG_CUDA(cudaEventRecord(ev[0], st.s));
@@ -275,13 +255,12 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
     if (ptotal) {
         std::vector<fe> pv(K * ptotal);
         parallel_proofs(K, [&](size_t k) {
-            for (const Run &r : runs)
-                for (size_t c = r.c0; c < r.c1; c++)
-                    memcpy(&pv[K * r.off + (k * (r.c1 - r.c0) + c - r.c0) * r.P], airs[k].periodic[c].values.data(), r.P * sizeof(fe));
+            for (const PeriodicRun &r : pr.runs)
+                for (size_t c = r.c0; c < r.c1; c++) memcpy(&pv[r.at(c, K, k)], airs[k].periodic[c].values.data(), r.P * sizeof(fe));
         });
         d_pvals.reserve(K * ptotal); d_pcoef.reserve(K * ptotal); d_ptab.reserve(K * ptotal * ce);
         CSG_CUDA(cudaMemcpyAsync(d_pvals.p, pv.data(), pv.size() * sizeof(fe), cudaMemcpyHostToDevice, st.s));
-        for (const Run &r : runs) {
+        for (const PeriodicRun &r : pr.runs) {
             const size_t cols = K * (r.c1 - r.c0);
             intt_columns(roots, ntt, d_pvals.p + K * r.off, r.P, d_pcoef.p + K * r.off, r.P, cols, ilog2(r.P), st);
             std::vector<fe> shifts(ce);
@@ -322,54 +301,24 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
         ConsArgs &A = T[0];
         memset(&A, 0, sizeof A);
         A.ext_degree = 1;
-        A.logn = logn; A.ncosets = (unsigned)ce; A.col_stride = n; A.width = (unsigned)w;
-        A.g_last = f63::pow(g, n - 1);
-        A.nconstraints = (unsigned)nc; A.ngroups = (unsigned)tg.adj.size();
-        for (size_t i = 0; i < nc; i++) A.group[i] = tg.group_of[i];
-        for (size_t gi = 0; gi < tg.adj.size(); gi++) A.adj_mod[gi] = tg.adj[gi] % n;
-        A.nbgroups = (unsigned)bg.groups.size(); A.nassertions = (unsigned)na;
-        for (size_t gi = 0; gi < bg.groups.size(); gi++) { A.b_adj_mod[gi] = bg.groups[gi].adj % n; A.b_steps[gi] = bg.groups[gi].num_steps; A.b_offset[gi] = bg.groups[gi].offset; }
-        for (size_t kc = 0; kc < ce; kc++) {
-            const fe s = ce_shift[kc];
-            A.lde_coset_stride[kc] = (unsigned long long)(kc * (b / ce)) * K * tw;
-            A.shift[kc] = s;
-            A.zinv[kc] = inv(sub(f63::pow(s, n), ONE));
-            for (size_t gi = 0; gi < tg.adj.size(); gi++) A.shift_adj[kc][gi] = f63::pow(s, tg.adj[gi]);
-            for (size_t gi = 0; gi < bg.groups.size(); gi++) { A.b_shift_adj[kc][gi] = f63::pow(s, bg.groups[gi].adj); A.b_shift_steps[kc][gi] = f63::pow(s, bg.groups[gi].num_steps); }
-        }
-        const fe g_inv = inv(g);
-        for (size_t i = 0; i < na; i++) {
-            const Assertion &s = air.assertions[i];
-            A.a_col[i] = s.column; A.a_group[i] = bg.group_of[i];
-            A.a_poly_len[i] = (unsigned)s.values.size();
-            A.a_xoff[i] = s.first_step ? f63::pow(g_inv, s.first_step) : ONE;
-        }
-        A.nperiodic = (unsigned)air.periodic.size();
-        A.ptab_coset_stride = K * ptotal;
-        for (const Run &r : runs) for (size_t c = r.c0; c < r.c1; c++) A.pmask[c] = (unsigned)(r.P - 1);
+        std::vector<size_t> lde_block(ce);
+        for (size_t kc = 0; kc < ce; kc++) lde_block[kc] = kc * (b / ce);
+        fill_domain_args(A, air, tg, bg, n, ce_shift, lde_block, K * tw);
     }
     std::vector<fe> apoly(std::max<size_t>(K * npoly, 1));
     parallel_proofs(K, [&](size_t k) {
         ProofState &p = ps[k];
-        p.coin.reseed(roots_h[k].data());
         memcpy(p.trace_root, roots_h[k].data(), 32);
+        const ProofTranscript::ConstraintCoefficients cc = p.tr.constraint_coefficients(p.trace_root, nc, na);
         ConsArgs &A = T[k];
         if (k) memcpy(&A, &T[0], sizeof A);
-        for (size_t i = 0; i < nc; i++) { A.alpha[i] = p.coin.draw(); A.beta[i] = p.coin.draw(); }
-        for (size_t i = 0; i < na; i++) { A.a_alpha[i] = p.coin.draw(); A.a_beta[i] = p.coin.draw(); }
+        for (size_t i = 0; i < nc; i++) { A.alpha[i] = cc.transition[2 * i].c[0]; A.beta[i] = cc.transition[2 * i + 1].c[0]; }
+        for (size_t i = 0; i < na; i++) { A.a_alpha[i] = cc.boundary[2 * i].c[0]; A.a_beta[i] = cc.boundary[2 * i + 1].c[0]; }
         fill_rescue_tables(air_id, A);
-        size_t po = k * npoly;
-        for (size_t i = 0; i < na; i++) {
-            const Assertion &s = airs[k].assertions[i];
-            A.a_value[i] = s.values[0];
-            A.a_poly_off[i] = po;
-            if (s.values.size() > 1) {
-                const std::vector<fe> c = interpolate_host(s.values);
-                std::copy(c.begin(), c.end(), apoly.begin() + po);
-                po += c.size();
-            }
-        }
-        for (const Run &r : runs) for (size_t c = r.c0; c < r.c1; c++) A.poff[c] = (unsigned)(K * r.off + (k * (r.c1 - r.c0) + c - r.c0) * r.P);
+        std::vector<fe> polys;
+        fill_assertion_values(A, airs[k], k * npoly, polys);
+        std::copy(polys.begin(), polys.end(), apoly.begin() + k * npoly);
+        fill_periodic_args(A, pr, K, k);
     });
     host_mark("draw coefficients, constraint arguments");
     d_cargs.reserve(K); d_apoly.reserve(apoly.size());
@@ -386,10 +335,7 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
     {
         std::vector<fe> sinv(K * ce);
         for (size_t kc = 0; kc < ce; kc++) { const fe s = inv(ce_shift[kc]); for (size_t k = 0; k < K; k++) sinv[k * ce + kc] = s; }
-        std::vector<fe> mat(ce * ce);
-        const fe off_n_inv = inv(f63::pow(to_mont(GENERATOR), n)), ce_inv = inv(to_mont(ce)), w_ce_inv = inv(root_of_unity(ilog2(ce)));
-        for (size_t t = 0; t < ce; t++)
-            for (size_t k = 0; k < ce; k++) mat[t * ce + k] = mul(mul(f63::pow(off_n_inv, t), ce_inv), f63::pow(w_ce_inv, (k * t) % ce));
+        const std::vector<fe> mat = composition_matrix(n, ce);
         d_e.reserve(K * ce * n); d_cpolys.reserve(K * ce * n); d_clde.reserve(b * K * ce * n);
         coset_intt_columns(roots, ntt, d_comb.p, n, d_e.p, n, logn, sinv.data(), K * ce, st);
         composition_columns_many(d_e.p, d_cpolys.p, n, (unsigned)ce, mat.data(), K, st);
@@ -408,9 +354,8 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
         std::vector<fe> pts(K * 6);   // per proof: (z, z^256), (zg, zg^256); then per proof (z^ce, (z^ce)^256)
         parallel_proofs(K, [&](size_t k) {
             ProofState &p = ps[k];
-            p.coin.reseed(roots_h[k].data());
             memcpy(p.comp_root, roots_h[k].data(), 32);
-            p.z = p.coin.draw();
+            p.z = p.tr.ood_point(p.comp_root).c[0];
             const fe zs[3] = {p.z, mul(p.z, g), f63::pow(p.z, ce)};
             for (int j = 0; j < 2; j++) { pts[k * 4 + 2 * j] = zs[j]; pts[k * 4 + 2 * j + 1] = f63::pow(zs[j], 256); }
             pts[K * 4 + 2 * k] = zs[2]; pts[K * 4 + 2 * k + 1] = f63::pow(zs[2], 256);
@@ -432,22 +377,11 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
             p.ood_cur.resize(w); p.ood_next.resize(w); p.ood_comp.resize(ce);
             for (size_t c = 0; c < w; c++) { p.ood_cur[c] = sum(((k * w + c) * 2) * nblk); p.ood_next[c] = sum(((k * w + c) * 2 + 1) * nblk); }
             for (size_t r = 0; r < ce; r++) p.ood_comp[r] = sum(K * w * 2 * nblk + (k * ce + r) * nblk);
-            uint8_t dg[32];
-            hash_elements_host(hf, p.ood_cur.data(), w, dg); p.coin.reseed(dg);
-            hash_elements_host(hf, p.ood_next.data(), w, dg); p.coin.reseed(dg);
-            hash_elements_host(hf, p.ood_comp.data(), ce, dg); p.coin.reseed(dg);
-            // DEEP coefficients: (alpha, beta) per trace column (a third draw is discarded), one per composition column, lambda, mu
-            DeepArgs &a = dargs[k];
-            a = DeepArgs{};
+            const ProofTranscript::DeepCoefficients dc = p.tr.deep_coefficients(p.ood_cur.data(), p.ood_next.data(), w, p.ood_comp.data(), ce);
             fe *ct = &coef[k * 2 * w], *cc = &coef[K * 2 * w + k * ce];
-            for (size_t c = 0; c < w; c++) { ct[c] = p.coin.draw(); ct[w + c] = p.coin.draw(); (void)p.coin.draw(); }
-            for (size_t r = 0; r < ce; r++) cc[r] = p.coin.draw();
-            a.lambda = p.coin.draw(); a.mu = p.coin.draw();
-            a.z = p.z; a.zg = mul(p.z, g); a.zm = f63::pow(p.z, ce);
-            for (size_t c = 0; c < w; c++) { a.az = add(a.az, mul(ct[c], p.ood_cur[c])); a.bzg = add(a.bzg, mul(ct[w + c], p.ood_next[c])); }
-            for (size_t r = 0; r < ce; r++) a.czm = add(a.czm, mul(cc[r], p.ood_comp[r]));
-            a.ncosets = (unsigned)b;
-            for (size_t s = 0; s < b; s++) a.shift[s] = lde_shift[s];
+            for (size_t c = 0; c < w; c++) { ct[c] = dc.trace[2 * c].c[0]; ct[w + c] = dc.trace[2 * c + 1].c[0]; }
+            for (size_t r = 0; r < ce; r++) cc[r] = dc.comp[r].c[0];
+            dargs[k] = deep_args(p.z, g, p.ood_cur, p.ood_next, p.ood_comp, ct, cc, dc.lambda.c[0], dc.mu.c[0], lde_shift.data(), b);
         });
         host_mark("deep coefficients");
         // ---------------------------------------------------------------- stage 6: DEEP composition
@@ -476,20 +410,10 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
         parallel_proofs(K, [&](size_t k) {
             ProofState &p = ps[k];
             memcpy(p.fri_roots[l].data(), roots_h[k].data(), 32);
-            p.coin.reseed(roots_h[k].data());
-            alphas[k] = p.coin.draw();
+            alphas[k] = p.tr.fri_alpha(p.fri_roots[l].data()).c[0];
         });
         if (l + 1 == nlayers) break;
-        const unsigned logm = ilog2(mm);
-        FoldArgs a{};
-        a.offset_inv = inv(to_mont(GENERATOR));
-        const fe w_inv = inv(root_of_unity(logm));
-        a.zeta_inv = f63::pow(w_inv, q); a.quarter = inv(to_mont(4));
-        a.logm = logm; a.logW = roots.logn;
-        if (logm > roots.logn) {
-            if (logm - roots.logn > 5) throw std::runtime_error("FRI layer too large for the root table");
-            for (unsigned i = 0; i < (1u << (logm - roots.logn)); i++) a.small[i] = f63::pow(w_inv, i);
-        }
+        const FoldArgs a = fold_args(mm, roots.logn);
         fri_evals[l + 1]->reserve(K * q);
         CSG_CUDA(cudaMemcpyAsync(d_args.p, alphas.data(), K * sizeof(fe), cudaMemcpyHostToDevice, st.s));
         fri_fold4_many(layer[l], mm, roots.W.p, a, d_args.p, K, fri_evals[l + 1]->p, st);
@@ -503,11 +427,8 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
     const size_t m_last = layer_m[nlayers - 1];
     parallel_proofs(K, [&](size_t k) {
         ProofState &p = ps[k];
-        uint64_t nonce = 1;
-        while (p.coin.check_leading_zeros(nonce) < o->grinding_factor) nonce++;
-        p.coin.reseed_with_int(nonce);
-        p.nonce = nonce;
-        p.pos = p.coin.draw_integers(nq, lde_n);
+        p.nonce = p.tr.grind(o->grinding_factor);
+        p.pos = p.tr.query_positions(nq, lde_n);
         // row jobs and digest jobs with offsets local to the proof
         auto plan = [&](Opening &op, const fe *data, unsigned width, unsigned ncosets, size_t coset_stride, size_t col_stride, const uint32_t *nodes,
                         size_t nleaves, const std::vector<size_t> &pos) {
@@ -611,13 +532,9 @@ void ManyProver::prove(Stream &st, int air_id, size_t K, ManyTraces traces, int 
     }
     tm.kernel_launches = st.launches - launches0;
     tm.total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    if (host_trace) {
-        host_mark("copy out");
-        double prev = 0;
-        fprintf(stderr, "[csg host trace] batch of %zu x (%zu x %zu), %llu launches; constraint arguments: %zu x %zu B up in %.3f ms\n", K, w, n,
+    host_mark("copy out");
+    trace.print("[csg host trace] batch of %zu x (%zu x %zu), %llu launches; constraint arguments: %zu x %zu B up in %.3f ms\n", K, w, n,
                 (unsigned long long)tm.kernel_launches, K, sizeof(ConsArgs), cargs_ms);
-        for (auto &mk : trace.marks) { fprintf(stderr, "  %-36s +%8.1f us  (at %8.1f)\n", mk.first, mk.second - prev, mk.second); prev = mk.second; }
-    }
 }
 
 }  // namespace csg

@@ -178,7 +178,11 @@ int csg_fri_remainder(csg_ctx *ctx, uint64_t *out, size_t cap, size_t *len) {
         ctx->need(S_DEEP, "the DEEP composition must be computed first");
         const FriLayer &L = *ctx->fri[ctx->nfri - 1];
         if (cap < L.m * ctx->d) throw ArgError("remainder buffer too small");
-        std::vector<uint64_t> rem = ctx->remainder();
+        csg_ctx::OpenBatch B;
+        ctx->plan_remainder(B, L);
+        std::vector<uint64_t> rem;
+        std::vector<uint8_t> digs;
+        ctx->run_openings(B, rem, digs);
         memcpy(out, rem.data(), rem.size() * 8);
         *len = rem.size();
     });
@@ -193,27 +197,33 @@ static std::vector<size_t> checked_positions(const uint64_t *positions, size_t n
     if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end()) throw ArgError("query positions must be distinct");
     return pos;
 }
-static void copy_opening(const std::vector<uint64_t> &r, const std::vector<uint8_t> &p, uint64_t *rows, uint8_t *paths, size_t cap, size_t *paths_len) {
+// fetches the one opening planned in B: its rows, and its Merkle paths as BatchMerkleProof::serialize_nodes() writes them
+static void copy_opening(csg_ctx *ctx, const csg_ctx::OpenBatch &B, const Opening &o, uint64_t *rows, uint8_t *paths, size_t cap, size_t *paths_len) {
+    std::vector<uint64_t> r;
+    std::vector<uint8_t> digs;
+    ctx->run_openings(B, r, digs);   // first: the ranks of a sharded proof sum their rows and paths in it
     if (!rows || !paths || !paths_len) throw ArgError("null output");
-    if (p.size() > cap) throw ArgError("path buffer too small");
-    memcpy(rows, r.data(), r.size() * 8);
-    memcpy(paths, p.data(), p.size());
-    *paths_len = p.size();
+    Bytes p;
+    write_paths(p, o, digs.data());
+    if (p.v.size() > cap) throw ArgError("path buffer too small");
+    memcpy(rows, r.data() + o.rows_off, o.rows_len * 8);
+    memcpy(paths, p.v.data(), p.v.size());
+    *paths_len = p.v.size();
 }
 int csg_open_trace(csg_ctx *ctx, const uint64_t *positions, size_t npos, uint64_t *rows, uint8_t *paths, size_t cap, size_t *paths_len) {
     return guarded(ctx, [&] {
         ctx->need(S_COMMITTED, "the trace must be committed first");
-        std::vector<size_t> pos = checked_positions(positions, npos, ctx->lde_n);
-        const size_t w = ctx->air.width;
-        copy_opening(ctx->open_rows(ctx->d_lde.p, (unsigned)w, (unsigned)ctx->b, w * ctx->n, ctx->n, pos, true), ctx->open_paths(ctx->d_tnodes, ctx->lde_n, pos, ctx->subtrees() ? &ctx->d_ttop : nullptr), rows, paths, cap, paths_len);
+        csg_ctx::OpenBatch B;
+        const Opening o = ctx->plan_trace_opening(B, checked_positions(positions, npos, ctx->lde_n));
+        copy_opening(ctx, B, o, rows, paths, cap, paths_len);
     });
 }
 int csg_open_composition(csg_ctx *ctx, const uint64_t *positions, size_t npos, uint64_t *rows, uint8_t *paths, size_t cap, size_t *paths_len) {
     return guarded(ctx, [&] {
         ctx->need(S_COMPOSED, "the composition polynomial must be committed first");
-        std::vector<size_t> pos = checked_positions(positions, npos, ctx->lde_n);
-        const size_t cw = ctx->ce * ctx->d;
-        copy_opening(ctx->open_rows(ctx->d_clde.p, (unsigned)cw, (unsigned)ctx->b, cw * ctx->n, ctx->n, pos, true), ctx->open_paths(ctx->d_cnodes, ctx->lde_n, pos, ctx->subtrees() ? &ctx->d_ctop : nullptr), rows, paths, cap, paths_len);
+        csg_ctx::OpenBatch B;
+        const Opening o = ctx->plan_composition_opening(B, checked_positions(positions, npos, ctx->lde_n));
+        copy_opening(ctx, B, o, rows, paths, cap, paths_len);
     });
 }
 int csg_open_fri_layer(csg_ctx *ctx, size_t layer, const uint64_t *positions, size_t npos, uint64_t *rows, uint8_t *paths, size_t cap, size_t *paths_len) {
@@ -221,8 +231,9 @@ int csg_open_fri_layer(csg_ctx *ctx, size_t layer, const uint64_t *positions, si
         ctx->need(S_DEEP, "the DEEP composition must be computed first");
         if (layer >= ctx->nfri || !ctx->fri[layer]->committed) throw ArgError("no such committed FRI layer");
         const FriLayer &L = *ctx->fri[layer];
-        std::vector<size_t> pos = checked_positions(positions, npos, L.m / 4);
-        copy_opening(ctx->open_fri_rows(L, pos), ctx->open_paths(L.nodes, L.m / 4, pos), rows, paths, cap, paths_len);
+        csg_ctx::OpenBatch B;
+        const Opening o = ctx->plan_fri_opening(B, L, checked_positions(positions, npos, L.m / 4));
+        copy_opening(ctx, B, o, rows, paths, cap, paths_len);
     });
 }
 // debugging aid: number of elements >= p in an internal device buffer (0 = trace polys, 1 = LDE, 2 = periodic tables,

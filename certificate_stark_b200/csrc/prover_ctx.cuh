@@ -25,6 +25,7 @@
 #include "host/air_desc.hpp"
 #include "host/batch_plan.hpp"
 #include "host/proof_common.hpp"
+#include "host/stage_args.hpp"
 #include "host/transcript.hpp"
 #include "many/many.cuh"
 #include "ntt.cuh"
@@ -77,7 +78,7 @@ class Timer {   // device time of a stage, CUDA events on the proving stream; th
         used_++;
     }
     // the same for a pair of events recorded elsewhere (they must not be re-recorded before the flush)
-    void span(cudaEvent_t a, cudaEvent_t b, float *dst, bool add = false) { pending_.push_back({a, b, dst, add}); }
+    void span(cudaEvent_t a, cudaEvent_t b, float *dst) { pending_.push_back({a, b, dst, false}); }
     void zero(float *dst) { pending_.push_back({nullptr, nullptr, dst, false}); }   // *dst = 0, in order with the spans
     bool crowded() const { return pending_.size() >= 256; }
     void discard() { pending_.clear(); used_ = 0; }   // nobody asked for the times of the previous proof
@@ -275,19 +276,14 @@ struct csg_ctx {
         d = (int)o->field_extension;
         if (d > 1) xk = ext_consts();
         n = trace_len; logn = ilog2(n); b = o->blowup_factor; ce = air.ce_blowup(); lde_n = n * b;
-        if (ce > b) throw ArgError("blowup factor is smaller than the constraint evaluation blowup of this AIR");
+        tg = transition_groups(air);
+        bg = boundary_groups(air);
+        try { check_air_shape(air, tg, bg, n, *o); } catch (const std::invalid_argument &e) { throw ArgError(e.what()); }
         G = comm ? (size_t)comm->world : 1; rank = comm ? (size_t)comm->rank : 0;
         csg_shard_plan plan;
         if (!shard_plan(rank, G, b, ce, air.width, &plan)) throw ArgError("the number of ranks of a sharded proof must divide the blowup factor");
         bl = plan.num_cosets; k0 = plan.first_coset;
         if (logn > 22) throw ArgError("trace length above 2^22 is not supported");
-        try { check_remainder(lde_n, *o); } catch (const std::invalid_argument &e) { throw ArgError(e.what()); }
-        if (air.num_constraints() > (size_t)CONS_MAX_CONSTRAINTS || air.periodic.size() > (size_t)CONS_MAX_PERIODIC ||
-            air.assertions.size() > (size_t)CONS_MAX_ASSERTIONS)
-            throw ArgError("AIR exceeds the compiled table sizes");
-        tg = transition_groups(air);
-        bg = boundary_groups(air);
-        if (tg.adj.size() > (size_t)CONS_MAX_GROUPS || bg.groups.size() > (size_t)CONS_MAX_BGROUPS) throw ArgError("too many constraint groups");
         roots.build(logn, st);
         const fe offset = to_mont(GENERATOR), w_lde = root_of_unity(ilog2(lde_n));
         std::vector<fe> all_shift(b);
@@ -310,34 +306,20 @@ struct csg_ctx {
         cargs_domain_ready = false;
         ConsArgs &A = *h_cargs;
         memset(&A, 0, sizeof A);
-        const size_t np = air.periodic.size();
-        A.nperiodic = (unsigned)np;
-        size_t total = 0;
-        for (size_t c = 0; c < np; c++) {
-            const size_t P = air.periodic[c].values.size();
-            if (P == 0 || (P & (P - 1)) || P > n) throw ArgError("periodic column length must be a power of two dividing the trace length");
-            A.poff[c] = (unsigned)total; A.pmask[c] = (unsigned)(P - 1);
-            total += P;
-        }
-        A.ptab_coset_stride = total;
-        d_ptab.reserve((total ? total : 1) * (cel ? cel : 1));
-        std::vector<bool> done(np, false);
+        const PeriodicRuns pr = periodic_runs(air);
+        fill_periodic_args(A, pr, 1, 0);
+        d_ptab.reserve((pr.total ? pr.total : 1) * (cel ? cel : 1));
         DBuf<fe> vals, coef;
-        for (size_t c0 = 0; c0 < np; c0++) {
-            if (done[c0]) continue;
-            const size_t P = air.periodic[c0].values.size();
-            // columns of this period that are contiguous in the table starting at c0
-            size_t c1 = c0;
-            while (c1 < np && air.periodic[c1].values.size() == P) { done[c1] = true; c1++; }
-            const size_t nc = c1 - c0;
+        for (const PeriodicRun &r : pr.runs) {
+            const size_t P = r.P, nc = r.c1 - r.c0;
             std::vector<fe> host(nc * P);
-            for (size_t c = c0; c < c1; c++) memcpy(&host[(c - c0) * P], air.periodic[c].values.data(), P * sizeof(fe));
+            for (size_t c = r.c0; c < r.c1; c++) memcpy(&host[(c - r.c0) * P], air.periodic[c].values.data(), P * sizeof(fe));
             vals.reserve(nc * P); coef.reserve(nc * P);
             CSG_CUDA(cudaMemcpyAsync(vals.p, host.data(), nc * P * sizeof(fe), cudaMemcpyHostToDevice, st.s));
             intt_columns(roots, ntt, vals.p, P, coef.p, P, nc, ilog2(P), st);
             std::vector<fe> shifts(cel);
             for (size_t kc = 0; kc < cel; kc++) shifts[kc] = f63::pow(ce_shift[kc], n / P);
-            if (cel) coset_ntt_columns(roots, ntt, coef.p, P, d_ptab.p + A.poff[c0], P, total, nc, ilog2(P), shifts.data(), cel, st);
+            if (cel) coset_ntt_columns(roots, ntt, coef.p, P, d_ptab.p + r.off, P, pr.total, nc, ilog2(P), shifts.data(), cel, st);
             CSG_CUDA(cudaStreamSynchronize(st.s));   // host staging vector goes out of scope
         }
     }
@@ -641,55 +623,22 @@ struct csg_ctx {
     }
 
     // ------------------------------------------------------------------------------------------ stage 3
-    // plane: which component of the E-valued coefficients these are (0 for the base field); the merged column of component j
-    // lands in d_comb[j][ce coset][row]
-    void eval_constraints(const fe *t_ab, const fe *b_ab, int plane = 0, bool all_components = false) {
+    // with a field extension, components 1.. of the coefficients are in h_cargs already (eval_constraints_x); the merged column of
+    // component j lands in d_comb[j][ce coset][row]
+    void eval_constraints(const fe *t_ab, const fe *b_ab) {
         need(S_COMMITTED, "the trace must be committed first");
         Timer &t = stage_timer;
         t.start(st);
         ConsArgs &A = *h_cargs;
-        A.ext_degree = all_components ? (unsigned)d : 1;
-        for (size_t i = 0; i < air.num_constraints(); i++) { A.alpha[i] = t_ab[2 * i]; A.beta[i] = t_ab[2 * i + 1]; A.group[i] = tg.group_of[i]; }
-        A.nconstraints = (unsigned)air.num_constraints(); A.ngroups = (unsigned)tg.adj.size();
-        fill_rescue_tables(air.id, A);
-        for (size_t i = 0; i < air.assertions.size(); i++) { A.a_alpha[i] = b_ab[2 * i]; A.a_beta[i] = b_ab[2 * i + 1]; }
-        host_mark("  cons: coefficient tables");
         if (!cargs_domain_ready) {
             // everything that depends on the AIR, the domain and the public inputs only: computed for the first proof after
             // csg_set_air and kept (some 150 host exponentiations and the assertion polynomials -- a fifth of the host time of
             // a one-transaction proof)
-            const fe g = root_of_unity(logn);
-            A.logn = logn; A.ncosets = (unsigned)cel; A.col_stride = n; A.width = air.width;
-            A.g_last = f63::pow(g, n - 1);
-            for (size_t gi = 0; gi < tg.adj.size(); gi++) A.adj_mod[gi] = tg.adj[gi] % n;
-            A.nbgroups = (unsigned)bg.groups.size(); A.nassertions = (unsigned)air.assertions.size();
-            for (size_t gi = 0; gi < bg.groups.size(); gi++) {
-                A.b_adj_mod[gi] = bg.groups[gi].adj % n; A.b_steps[gi] = bg.groups[gi].num_steps; A.b_offset[gi] = bg.groups[gi].offset;
-            }
-            for (size_t kc = 0; kc < cel; kc++) {
-                const fe s = ce_shift[kc];
-                A.lde_coset_stride[kc] = (unsigned long long)((kc0 + kc) * (b / ce) - k0) * air.width * n;
-                A.shift[kc] = s;
-                A.zinv[kc] = inv(sub(f63::pow(s, n), ONE));
-                for (size_t gi = 0; gi < tg.adj.size(); gi++) A.shift_adj[kc][gi] = f63::pow(s, tg.adj[gi]);
-                for (size_t gi = 0; gi < bg.groups.size(); gi++) {
-                    A.b_shift_adj[kc][gi] = f63::pow(s, bg.groups[gi].adj);
-                    A.b_shift_steps[kc][gi] = f63::pow(s, bg.groups[gi].num_steps);
-                }
-            }
-            // assertion values; a sequence becomes its interpolating polynomial, evaluated in-kernel at x * g^-first_step
+            std::vector<size_t> lde_block(cel);
+            for (size_t kc = 0; kc < cel; kc++) lde_block[kc] = (kc0 + kc) * (b / ce) - k0;
+            fill_domain_args(A, air, tg, bg, n, ce_shift, lde_block, air.width * n);
             std::vector<fe> polys;
-            const fe g_inv = inv(g);
-            for (size_t i = 0; i < air.assertions.size(); i++) {
-                const Assertion &s = air.assertions[i];
-                A.a_col[i] = s.column; A.a_group[i] = bg.group_of[i];
-                A.a_value[i] = s.values[0]; A.a_poly_len[i] = (unsigned)s.values.size(); A.a_poly_off[i] = polys.size();
-                A.a_xoff[i] = s.first_step ? f63::pow(g_inv, s.first_step) : ONE;
-                if (s.values.size() > 1) {
-                    std::vector<fe> c = interpolate_host(s.values);
-                    polys.insert(polys.end(), c.begin(), c.end());
-                }
-            }
+            fill_assertion_values(A, air, 0, polys);
             d_apoly.reserve(polys.size() ? polys.size() : 1);
             if (!polys.empty()) {   // pageable source: wait for the copy before `polys` goes away
                 CSG_CUDA(cudaMemcpyAsync(d_apoly.p, polys.data(), polys.size() * sizeof(fe), cudaMemcpyHostToDevice, st.s));
@@ -697,11 +646,15 @@ struct csg_ctx {
             }
             cargs_domain_ready = true;
         }
+        A.ext_degree = (unsigned)d;
+        for (size_t i = 0; i < air.num_constraints(); i++) { A.alpha[i] = t_ab[2 * i]; A.beta[i] = t_ab[2 * i + 1]; }
+        fill_rescue_tables(air.id, A);
+        for (size_t i = 0; i < air.assertions.size(); i++) { A.a_alpha[i] = b_ab[2 * i]; A.a_beta[i] = b_ab[2 * i + 1]; }
+        host_mark("  cons: coefficient tables");
         d_cargs.reserve(1);
         CSG_CUDA(cudaMemcpyAsync(d_cargs.p, &A, sizeof A, cudaMemcpyHostToDevice, st.s));
-        const size_t comb_plane = (cel ? cel : 1) * n;
-        d_comb.reserve(comb_plane * d);
-        d_parts.reserve(constraint_scratch_elements(air.id, n, cel ? cel : 1) * (all_components ? d : 1));
+        d_comb.reserve((cel ? cel : 1) * n * d);
+        d_parts.reserve(constraint_scratch_elements(air.id, n, cel ? cel : 1) * d);
         host_mark("  cons: args upload, scratch");
         if (!cons_ev[0]) for (auto &e : cons_ev) CSG_CUDA(cudaEventCreate(&e));
         // the low-degree splits interpolate across the even cosets: alone, or with an exchange when every rank owns whole pairs
@@ -712,33 +665,23 @@ struct csg_ctx {
             xch.buf = d_xch.p; xch.buf_elems = d_xch.n;
         }
         const SplitExchange *px = split && G > 1 ? &xch : nullptr;
-        if (cel && all_components) csg::eval_constraints_ext(air.id, d_cargs.p, A, d_lde.p, roots.W.p, d_ptab.p, d_apoly.p, d_parts.p, d_comb.p, st, cons_ev,
-                                                             split ? &roots : nullptr, split ? &ntt : nullptr, px);
-        else if (cel) csg::eval_constraints(air.id, d_cargs.p, A, d_lde.p, roots.W.p, d_ptab.p, d_apoly.p, d_parts.p, d_comb.p + plane * comb_plane, st, cons_ev,
+        if (cel && d > 1) csg::eval_constraints_ext(air.id, d_cargs.p, A, d_lde.p, roots.W.p, d_ptab.p, d_apoly.p, d_parts.p, d_comb.p, st, cons_ev,
+                                                    split ? &roots : nullptr, split ? &ntt : nullptr, px);
+        else if (cel) csg::eval_constraints(air.id, d_cargs.p, A, d_lde.p, roots.W.p, d_ptab.p, d_apoly.p, d_parts.p, d_comb.p, st, cons_ev,
                                             split ? &roots : nullptr, split ? &ntt : nullptr, px);
         else for (auto &e : cons_ev) CSG_CUDA(cudaEventRecord(e, st.s));
-        t.stop(st, &tm.constraints, plane != 0);   // (`polys` is pageable memory: its copy was staged before cudaMemcpyAsync returned)
-        tm.stage_launches[2] = plane ? tm.stage_launches[2] + t.launches : t.launches;
+        t.stop(st, &tm.constraints);   // (`polys` is pageable memory: its copy was staged before cudaMemcpyAsync returned)
+        tm.stage_launches[2] = t.launches;
         float *parts_ms[4] = {&tm.cons_rescue, &tm.cons_ecc_banks, &tm.cons_ecc_final, &tm.cons_rest};
-        for (int k = 0; k < 4; k++) t.span(cons_ev[k], cons_ev[k + 1], parts_ms[k], plane != 0);
-        t.span(cons_ev[1], cons_ev[5], &tm.cons_ecc_low, plane != 0);
-        if (d > 1 && !all_components) t.flush();   // evaluated plane by plane: the next plane records the same events again
-        if (plane + 1 == d || all_components) stage = S_EVALUATED;
+        for (int k = 0; k < 4; k++) t.span(cons_ev[k], cons_ev[k + 1], parts_ms[k]);
+        t.span(cons_ev[1], cons_ev[5], &tm.cons_ecc_low);
+        stage = S_EVALUATED;
     }
     // E-valued coefficients: the constraint values are base-field elements, so component j of the merged column is the same
-    // combination with component j of every coefficient -- d passes of the base-field evaluation
+    // combination with component j of every coefficient; one pass, every thread accumulates all d components (constraints_ext.cu)
     void eval_constraints_x(const xe *t_ab, const xe *b_ab) {
         const size_t nc = air.num_constraints(), na = air.assertions.size();
         std::vector<fe> tj(2 * nc), bj(2 * na + 2);
-        if (getenv("CSG_EXT_PASSES")) {   // A/B: one pass of the base-field kernels per component
-            for (int j = 0; j < d; j++) {
-                for (size_t i = 0; i < 2 * nc; i++) tj[i] = t_ab[i].c[j];
-                for (size_t i = 0; i < 2 * na; i++) bj[i] = b_ab[i].c[j];
-                eval_constraints(tj.data(), bj.data(), j);
-            }
-            return;
-        }
-        // one pass: every thread accumulates all d components (constraints_ext.cu)
         ConsArgs &A = *h_cargs;
         for (int j = 1; j < d; j++) {
             for (size_t i = 0; i < nc; i++) { A.alpha_x[j - 1][i] = t_ab[2 * i].c[j]; A.beta_x[j - 1][i] = t_ab[2 * i + 1].c[j]; }
@@ -746,7 +689,7 @@ struct csg_ctx {
         }
         for (size_t i = 0; i < 2 * nc; i++) tj[i] = t_ab[i].c[0];
         for (size_t i = 0; i < 2 * na; i++) bj[i] = b_ab[i].c[0];
-        eval_constraints(tj.data(), bj.data(), 0, true);
+        eval_constraints(tj.data(), bj.data());
     }
     // ------------------------------------------------------------------------------------------ stage 4
     void commit_composition(uint8_t root[32]) {
@@ -757,11 +700,7 @@ struct csg_ctx {
         std::vector<fe> sinv(cel);
         for (size_t kc = 0; kc < cel; kc++) sinv[kc] = inv(ce_shift[kc]);
         d_e.reserve(ce * n); d_cpolys.reserve(ce * d * n);
-        std::vector<fe> mat(ce * ce);
-        const fe off_n_inv = inv(f63::pow(to_mont(GENERATOR), n)), ce_inv = inv(to_mont(ce)), w_ce_inv = inv(root_of_unity(ilog2(ce)));
-        for (size_t tt = 0; tt < ce; tt++)
-            for (size_t k = 0; k < ce; k++)
-                mat[tt * ce + k] = mul(mul(f63::pow(off_n_inv, tt), ce_inv), f63::pow(w_ce_inv, (k * tt) % ce));
+        const std::vector<fe> mat = composition_matrix(n, ce);
         // component j of composition column r is the base-field column r*d + j: rows hash as ce elements of E
         for (int j = 0; j < d; j++) {
         const fe *comb = d_comb.p + (size_t)j * (cel ? cel : 1) * n;
@@ -823,16 +762,8 @@ struct csg_ctx {
         t.start(st);
         const size_t w = air.width;
         std::vector<fe> coef(2 * w);
-        DeepArgs a{};
-        a.z = z; a.zg = mul(z, root_of_unity(logn)); a.zm = f63::pow(z, ce);
-        for (size_t c = 0; c < w; c++) {
-            coef[c] = trace_ab[2 * c]; coef[w + c] = trace_ab[2 * c + 1];
-            a.az = add(a.az, mul(coef[c], ood_cur[c]));
-            a.bzg = add(a.bzg, mul(coef[w + c], ood_next[c]));
-        }
-        for (size_t r = 0; r < ce; r++) a.czm = add(a.czm, mul(comp_d[r], ood_comp[r]));
-        a.lambda = lambda; a.mu = mu; a.ncosets = (unsigned)bl;
-        for (size_t k = 0; k < bl; k++) a.shift[k] = lde_shift[k];
+        for (size_t c = 0; c < w; c++) { coef[c] = trace_ab[2 * c]; coef[w + c] = trace_ab[2 * c + 1]; }
+        const DeepArgs a = deep_args(z, root_of_unity(logn), ood_cur, ood_next, ood_comp, coef.data(), comp_d, lambda, mu, lde_shift.data(), bl);
         d_abc.reserve(3 * n); d_abc_lde.reserve(3 * n * bl); d_deep.reserve(lde_n);
         combine_polys(d_polys.p, n, w, n, coef.data(), 2, d_abc.p, n, scratch2, st);
         combine_polys(d_cpolys.p, n, ce, n, comp_d, 1, d_abc.p + 2 * n, n, scratch, st);
@@ -965,16 +896,8 @@ struct csg_ctx {
         Timer &t = stage_timer;
         t.start(st);
         const size_t m = L.m, q = m / 4;
-        const unsigned logm = ilog2(m);
-        FoldArgs a{};
-        a.alpha = alpha.c[0]; a.offset_inv = inv(to_mont(GENERATOR));
-        const fe w_inv = inv(root_of_unity(logm));
-        a.zeta_inv = f63::pow(w_inv, q); a.quarter = inv(to_mont(4));
-        a.logm = logm; a.logW = roots.logn;
-        if (logm > roots.logn) {
-            if (logm - roots.logn > 5) throw StateError("FRI layer too large for the root table");
-            for (unsigned i = 0; i < (1u << (logm - roots.logn)); i++) a.small[i] = f63::pow(w_inv, i);
-        }
+        FoldArgs a = fold_args(m, roots.logn);
+        a.alpha = alpha.c[0];
         if (fri.size() == nfri) fri.emplace_back(new FriLayer());
         FriLayer &N = *fri[nfri];
         N.owned.reserve(q * d);
@@ -986,63 +909,6 @@ struct csg_ctx {
     }
     size_t num_fri_folds() const { return csg::num_fri_folds(lde_n, opt); }
 
-    // ------------------------------------------------------------------------------------------ stage 9
-    void upload_positions(const std::vector<uint32_t> &p32) {
-        d_idx.reserve(std::max<size_t>(p32.size(), 4096));
-        // no wait here: every caller keeps p32 alive until it has downloaded what the positions select
-        CSG_CUDA(cudaMemcpyAsync(d_idx.p, p32.data(), p32.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st.s));
-    }
-    // rows (canonical, row-major) of a coset-major matrix at the given natural positions
-    // sharded (the LDE matrices of a split proof): every context gathers the rows of its own cosets, zeros elsewhere, and the
-    // row buffers are summed across the ranks
-    std::vector<uint64_t> open_rows(const fe *data, unsigned width, unsigned ncosets, size_t coset_stride, size_t col_stride, const std::vector<size_t> &pos,
-                                    bool sharded = false, unsigned sub = 1, size_t sub_stride = 0) {
-        std::vector<uint32_t> p32(pos.begin(), pos.end());
-        sharded = sharded && G > 1;
-        if (sharded) {
-            for (auto &p : p32) {
-                const size_t k = p % b, i = p / b;
-                p = (k >= k0 && k < k0 + bl) ? (uint32_t)((k - k0) + bl * i) : 0xFFFFFFFFu;
-            }
-            ncosets = (unsigned)bl;
-        }
-        upload_positions(p32);
-        std::vector<uint64_t> rows(pos.size() * width);
-        // d_io still holds the resident trace for re-proving; rows go through a separate small buffer
-        d_rows.reserve(std::max<size_t>(rows.size(), 1 << 16));
-        gather_rows(data, width, ncosets, coset_stride, col_stride, d_idx.p, pos.size(), d_rows.p, st, sub, sub_stride);
-        if (sharded) reduce_rows(d_rows.p, rows.size());
-        CSG_CUDA(cudaMemcpyAsync(rows.data(), d_rows.p, rows.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, st.s));
-        CSG_CUDA(cudaStreamSynchronize(st.s));
-        return rows;
-    }
-    // BatchMerkleProof::serialize_nodes() of the opening of `pos` in the tree `nodes` over nleaves leaves
-    // top != nullptr: `nodes` is this context's subtree of a sharded tree (commit_rows); the path nodes are summed across the ranks
-    std::vector<uint8_t> open_paths(const DBuf<uint32_t> &nodes, size_t nleaves, const std::vector<size_t> &pos, const DBuf<uint32_t> *top = nullptr) {
-        std::vector<std::vector<uint32_t>> slots = batch_opening_nodes(nleaves, pos);
-        std::vector<uint32_t> flat;
-        for (auto &s : slots) flat.insert(flat.end(), s.begin(), s.end());
-        if (top) for (auto &v : flat) v = tree_ref(v);
-        std::vector<uint8_t> dig(flat.size() * 32);
-        if (!flat.empty()) {
-            d_idx.reserve(std::max<size_t>(flat.size(), 4096));
-            d_dig.reserve(std::max<size_t>(flat.size() * 8, 8 * 4096));
-            CSG_CUDA(cudaMemcpyAsync(d_idx.p, flat.data(), flat.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st.s));
-            gather_digests(nodes.p, d_idx.p, flat.size(), d_dig.p, st, top ? top->p : nullptr);
-            if (top) reduce_rows((uint64_t *)d_dig.p, flat.size() * 4);
-            CSG_CUDA(cudaMemcpyAsync(dig.data(), d_dig.p, dig.size(), cudaMemcpyDeviceToHost, st.s));
-            CSG_CUDA(cudaStreamSynchronize(st.s));
-        }
-        std::vector<uint8_t> out;
-        out.push_back((uint8_t)slots.size());
-        size_t o = 0;
-        for (auto &s : slots) {
-            out.push_back((uint8_t)s.size());
-            out.insert(out.end(), dig.begin() + o * 32, dig.begin() + (o + s.size()) * 32);
-            o += s.size();
-        }
-        return out;
-    }
     // ------------------------------------------------------------------------------------------ the whole of Prover::prove
     void write_context(Bytes &w) const { write_proof_context(w, air.width, logn, opt); }
     // flattened components of E elements (serialisation / hashing order)
@@ -1054,113 +920,84 @@ struct csg_ctx {
     void prove_loaded(uint8_t **proof, size_t *proof_len, const uint64_t *host = nullptr, int host_repr = CSG_REPR_CANONICAL, const uint64_t *const *host_cols = nullptr) {
         if (!host && !host_cols) need(S_TRACE, "csg_load_trace must be called first");
         auto t0 = std::chrono::steady_clock::now();
-        // CSG_HOST_TRACE: host clock at the stage boundaries of this call, printed to stderr (where the time of a small proof
-        // goes: launches, round trips of the Fiat-Shamir transcript, host arithmetic)
-        static const bool host_trace = getenv("CSG_HOST_TRACE") != nullptr;
-        HostTrace trace{t0, {}};
-        struct TraceScope { bool on; TraceScope(bool o, HostTrace *t) : on(o) { if (on) g_host_trace = t; } ~TraceScope() { if (on) g_host_trace = nullptr; } } trace_scope(host_trace, &trace);
-        auto mark = [&](const char *what) { host_mark(what); };
+        HostTraceScope trace(t0);
         const unsigned long long launches0 = st.launches;
         stage_timer.discard(); query_timer.discard();
         comm_used = 0;
-        const int hf = (int)opt.hash_fn;
         const size_t w = air.width, nc = air.num_constraints(), na = air.assertions.size();
-        Bytes seed;
-        for (uint64_t v : air.pub_inputs) seed.u64(v);
-        write_context(seed);
-        Coin coin(hf, seed.v.data(), seed.v.size());
+        Bytes context;
+        write_context(context);
+        ProofTranscript tr((int)opt.hash_fn, d, air.pub_inputs.data(), air.pub_inputs.size(), context.v.data(), context.v.size());
         auto base = [](const std::vector<xe> &v) { std::vector<fe> o; for (const xe &e : v) o.push_back(e.c[0]); return o; };
 
         uint8_t trace_root[32], comp_root[32];
-        mark("setup");
+        host_mark("setup");
         extend_and_commit_trace(trace_root, host, host_repr, host_cols);
-        mark("extend+commit trace");
-        coin.reseed(trace_root);
-        std::vector<xe> t_ab(2 * nc), b_ab(2 * na + 2, x_zero());
-        for (size_t i = 0; i < 2 * nc; i++) t_ab[i] = coin.draw_x(d);
-        for (size_t i = 0; i < 2 * na; i++) b_ab[i] = coin.draw_x(d);
-        mark("draw coefficients");
-        if (d == 1) eval_constraints(base(t_ab).data(), base(b_ab).data());
-        else eval_constraints_x(t_ab.data(), b_ab.data());
-        mark("constraints (enqueue)");
+        host_mark("extend+commit trace");
+        const ProofTranscript::ConstraintCoefficients cc = tr.constraint_coefficients(trace_root, nc, na);
+        host_mark("draw coefficients");
+        if (d == 1) eval_constraints(base(cc.transition).data(), base(cc.boundary).data());
+        else eval_constraints_x(cc.transition.data(), cc.boundary.data());
+        host_mark("constraints (enqueue)");
         commit_composition(comp_root);
-        mark("composition + commit");
-        coin.reseed(comp_root);
+        host_mark("composition + commit");
 
-        const xe zz = coin.draw_x(d);
-        if (d == 1) {
-            ood(zz.c[0]);
-            xood_cur.clear(); xood_next.clear(); xood_comp.clear();
-            for (fe v : ood_cur) xood_cur.push_back(x_from(v));
-            for (fe v : ood_next) xood_next.push_back(x_from(v));
-            for (fe v : ood_comp) xood_comp.push_back(x_from(v));
-        } else ood_x(zz);
-        uint8_t dg[32];
-        hash_elements_host(hf, flat(xood_cur).data(), w * d, dg); coin.reseed(dg);
-        hash_elements_host(hf, flat(xood_next).data(), w * d, dg); coin.reseed(dg);
-        hash_elements_host(hf, flat(xood_comp).data(), ce * d, dg); coin.reseed(dg);
-        mark("out-of-domain frame");
-
-        std::vector<xe> dab(2 * w), dd(ce);
-        for (size_t c = 0; c < w; c++) { dab[2 * c] = coin.draw_x(d); dab[2 * c + 1] = coin.draw_x(d); (void)coin.draw_x(d); }
-        for (size_t r = 0; r < ce; r++) dd[r] = coin.draw_x(d);
-        const xe lambda = coin.draw_x(d), mu = coin.draw_x(d);
-        if (d == 1) deep(base(dab).data(), base(dd).data(), lambda.c[0], mu.c[0]);
-        else deep_x(dab.data(), dd.data(), lambda, mu);
-        mark("deep (enqueue)");
+        const xe zz = tr.ood_point(comp_root);
+        if (d == 1) ood(zz.c[0]);
+        else ood_x(zz);
+        const std::vector<fe> f_cur = d == 1 ? ood_cur : flat(xood_cur), f_next = d == 1 ? ood_next : flat(xood_next),
+                              f_comp = d == 1 ? ood_comp : flat(xood_comp);
+        const ProofTranscript::DeepCoefficients dc = tr.deep_coefficients(f_cur.data(), f_next.data(), w, f_comp.data(), ce);
+        host_mark("out-of-domain frame");
+        if (d == 1) deep(base(dc.trace).data(), base(dc.comp).data(), dc.lambda.c[0], dc.mu.c[0]);
+        else deep_x(dc.trace.data(), dc.comp.data(), dc.lambda, dc.mu);
+        host_mark("deep (enqueue)");
 
         const size_t nlayers = num_fri_folds() + 1;
         std::vector<std::vector<uint8_t>> fri_roots(nlayers, std::vector<uint8_t>(32));
         for (size_t l = 0; l < nlayers; l++) {
             fri_commit_layer(fri_roots[l].data());
-            coin.reseed(fri_roots[l].data());
-            const xe alpha = coin.draw_x(d);
+            const xe alpha = tr.fri_alpha(fri_roots[l].data());
             if (l + 1 < nlayers) fri_fold_x(alpha);
         }
-        mark("fri layers");
+        host_mark("fri layers");
 
         Timer &tq = query_timer;
         tq.start(st);
-        uint64_t nonce = 1;
-        while (coin.check_leading_zeros(nonce) < opt.grinding_factor) nonce++;
-        coin.reseed_with_int(nonce);
-        std::vector<size_t> pos = coin.draw_integers(opt.num_queries, lde_n);
-        mark("grinding + positions");
+        const uint64_t nonce = tr.grind(opt.grinding_factor);
+        const std::vector<size_t> pos = tr.query_positions(opt.num_queries, lde_n);
+        host_mark("grinding + positions");
 
         // every opening of the proof -- trace rows, composition rows, FRI layer rows, their Merkle paths, the remainder -- is
         // planned on the host first and fetched in ONE round trip (one index upload, a handful of gather launches, one download)
         OpenBatch B;
-        const size_t cw = ce * d;
-        const Opening o_trace = plan_opening(B, d_lde.p, (unsigned)w, (unsigned)b, w * n, n, 1, 0, true, d_tnodes.p, lde_n, pos, subtrees() ? d_ttop.p : nullptr);
-        const Opening o_comp = plan_opening(B, d_clde.p, (unsigned)cw, (unsigned)b, cw * n, n, 1, 0, true, d_cnodes.p, lde_n, pos, subtrees() ? d_ctop.p : nullptr);
+        const Opening o_trace = plan_trace_opening(B, pos);
+        const Opening o_comp = plan_composition_opening(B, pos);
         std::vector<Opening> o_fri;
         {
             std::vector<size_t> fp = pos;
             size_t domain = lde_n;
             for (size_t l = 0; l + 1 < nlayers; l++) {
                 fp = fold_positions(fp, domain);
-                const size_t q = domain / 4;
-                const FriLayer &L = *fri[l];
-                o_fri.push_back(plan_opening(B, L.evals, 4 * (unsigned)d, 1, 0, q, (unsigned)d, d == 1 ? 0 : L.m, false, L.nodes.p, q, fp));
-                domain = q;
+                o_fri.push_back(plan_fri_opening(B, *fri[l], fp));
+                domain /= 4;
             }
         }
         const FriLayer &last = *fri[nlayers - 1];
-        const size_t rem_off = B.rows_words, rem_len = last.m * d;
-        B.rows_words += rem_len;
+        const size_t rem_off = plan_remainder(B, last), rem_len = last.m * d;
         std::vector<uint64_t> rows;
         std::vector<uint8_t> digs;
-        mark("plan openings");
-        run_openings(B, rows, digs, last, rem_off);
-        mark("openings round trip");
+        host_mark("plan openings");
+        run_openings(B, rows, digs);
+        host_mark("openings round trip");
         Bytes pf;
         pf.v.reserve(256 * 1024);
         std::vector<const uint8_t *> fri_root_ptrs;
         for (auto &r : fri_roots) fri_root_ptrs.push_back(r.data());
-        write_proof(pf, (unsigned)w, logn, opt, trace_root, comp_root, fri_root_ptrs, o_trace, o_comp, o_fri, rows.data(), digs.data(), flat(xood_cur),
-                    flat(xood_next), flat(xood_comp), rem_off, rem_len, nonce);
+        write_proof(pf, (unsigned)w, logn, opt, trace_root, comp_root, fri_root_ptrs, o_trace, o_comp, o_fri, rows.data(), digs.data(), f_cur, f_next, f_comp,
+                    rem_off, rem_len, nonce);
         tq.stop(st, &tm.queries); tm.stage_launches[6] = tq.launches;
-        mark("serialise");
+        host_mark("serialise");
         tm.kernel_launches = st.launches - launches0;
         tm.comm = comm_ms();
         tm.total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1169,12 +1006,8 @@ struct csg_ctx {
         if (!*proof) throw std::bad_alloc();
         memcpy(*proof, pf.v.data(), pf.v.size());
         *proof_len = pf.v.size();
-        if (host_trace) {
-            mark("timers + copy out");
-            double prev = 0;
-            fprintf(stderr, "[csg host trace] %zu x %zu, %llu launches\n", (size_t)air.width, n, (unsigned long long)tm.kernel_launches);
-            for (auto &m : trace.marks) { fprintf(stderr, "  %-24s +%8.1f us  (at %8.1f)\n", m.first, m.second - prev, m.second); prev = m.second; }
-        }
+        host_mark("timers + copy out");
+        trace.print("[csg host trace] %zu x %zu, %llu launches\n", (size_t)air.width, n, (unsigned long long)tm.kernel_launches);
         stage = S_TRACE;   // the resident trace (d_io) can be proved again
     }
     // ---- batched openings
@@ -1185,6 +1018,8 @@ struct csg_ctx {
         std::vector<Rows> rows;
         std::vector<Digs> digs;
         size_t rows_words = 0, dig_count = 0, sharded_words = 0, sharded_digs = 0;   // sharded_*: leading parts summed across the ranks
+        const FriLayer *rem = nullptr;   // the remainder, if planned (plan_remainder), at rows[rem_off ..)
+        size_t rem_off = 0;
     };
     // rows of `data` at `pos` (sharded matrices first: their rows are summed across the ranks in one go) and the batch opening
     // of the same positions in the tree `nodes`
@@ -1211,39 +1046,41 @@ struct csg_ctx {
         B.digs.push_back(dj);
         return o;
     }
-    void run_openings(OpenBatch &B, std::vector<uint64_t> &rows, std::vector<uint8_t> &digs, const FriLayer &last, size_t rem_off) {
+    // the openings of the committed matrices: sharded ones first (plan_opening)
+    Opening plan_trace_opening(OpenBatch &B, const std::vector<size_t> &pos) {
+        return plan_opening(B, d_lde.p, (unsigned)air.width, (unsigned)b, air.width * n, n, 1, 0, true, d_tnodes.p, lde_n, pos, subtrees() ? d_ttop.p : nullptr);
+    }
+    Opening plan_composition_opening(OpenBatch &B, const std::vector<size_t> &pos) {
+        const size_t cw = ce * d;
+        return plan_opening(B, d_clde.p, (unsigned)cw, (unsigned)b, cw * n, n, 1, 0, true, d_cnodes.p, lde_n, pos, subtrees() ? d_ctop.p : nullptr);
+    }
+    // rows of 4 elements of E, each d components (planes of stride m)
+    Opening plan_fri_opening(OpenBatch &B, const FriLayer &L, const std::vector<size_t> &pos) {
+        const size_t q = L.m / 4;
+        return plan_opening(B, L.evals, 4 * (unsigned)d, 1, 0, q, (unsigned)d, d == 1 ? 0 : L.m, false, L.nodes.p, q, pos);
+    }
+    // the last FRI layer in natural order, canonical, components of an element adjacent: returns where it sits among the opened words
+    size_t plan_remainder(OpenBatch &B, const FriLayer &last) {
+        B.rem = &last; B.rem_off = B.rows_words;
+        B.rows_words += last.m * d;
+        return B.rem_off;
+    }
+    void run_openings(const OpenBatch &B, std::vector<uint64_t> &rows, std::vector<uint8_t> &digs) {
         d_idx.reserve(std::max<size_t>(B.idx.size(), 1 << 16));
         d_rows.reserve(std::max<size_t>(B.rows_words, 1 << 17));
         d_dig.reserve(std::max<size_t>(B.dig_count * 8, 8 << 16));
-        CSG_CUDA(cudaMemcpyAsync(d_idx.p, B.idx.data(), B.idx.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st.s));
+        if (!B.idx.empty()) CSG_CUDA(cudaMemcpyAsync(d_idx.p, B.idx.data(), B.idx.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st.s));
         for (auto &r : B.rows)
             gather_rows(r.data, r.width, r.ncosets, r.coset_stride, r.col_stride, d_idx.p + r.idx_off, r.npos, d_rows.p + r.rows_off, st, r.sub, r.sub_stride);
         if (B.sharded_words) reduce_rows(d_rows.p, B.sharded_words);
         for (auto &g : B.digs) gather_digests(g.nodes, d_idx.p + g.idx_off, g.count, d_dig.p + 8 * g.dig_off, st, g.top);
         if (B.sharded_digs) reduce_rows((uint64_t *)d_dig.p, B.sharded_digs * 4);
-        if (d == 1) from_montgomery(last.evals, d_rows.p + rem_off, last.m, st);
-        else planes_to_canonical(last.evals, last.m, last.m, d, d_rows.p + rem_off, st);
+        if (B.rem && d == 1) from_montgomery(B.rem->evals, d_rows.p + B.rem_off, B.rem->m, st);
+        else if (B.rem) planes_to_canonical(B.rem->evals, B.rem->m, B.rem->m, d, d_rows.p + B.rem_off, st);
         rows.resize(B.rows_words); digs.resize(B.dig_count * 32);
         CSG_CUDA(cudaMemcpyAsync(rows.data(), d_rows.p, rows.size() * 8, cudaMemcpyDeviceToHost, st.s));
         if (!digs.empty()) CSG_CUDA(cudaMemcpyAsync(digs.data(), d_dig.p, digs.size(), cudaMemcpyDeviceToHost, st.s));
         CSG_CUDA(cudaStreamSynchronize(st.s));
-    }
-    // opened rows of a FRI layer: 4 elements per row, each d components (planes of stride m)
-    std::vector<uint64_t> open_fri_rows(const FriLayer &L, const std::vector<size_t> &pos) {
-        const size_t q = L.m / 4;
-        if (d == 1) return open_rows(L.evals, 4, 1, 0, q, pos);
-        return open_rows(L.evals, 4 * d, 1, 0, q, pos, false, (unsigned)d, L.m);
-    }
-    // the last layer in natural order, canonical, components of an element adjacent
-    std::vector<uint64_t> remainder() {
-        const FriLayer &last = *fri[nfri - 1];
-        std::vector<uint64_t> rem(last.m * d);
-        d_rows.reserve(std::max<size_t>(rem.size(), 1 << 16));
-        if (d == 1) from_montgomery(last.evals, d_rows.p, last.m, st);
-        else planes_to_canonical(last.evals, last.m, last.m, d, d_rows.p, st);
-        CSG_CUDA(cudaMemcpyAsync(rem.data(), d_rows.p, rem.size() * 8, cudaMemcpyDeviceToHost, st.s));
-        CSG_CUDA(cudaStreamSynchronize(st.s));
-        return rem;
     }
 };
 
