@@ -25,6 +25,8 @@ HASH_BLAKE3_256, HASH_SHA3_256 = 2, 3
 FIELD_EXTENSION_NONE, FIELD_EXTENSION_QUADRATIC, FIELD_EXTENSION_CUBIC = 1, 2, 3
 REPR_CANONICAL, REPR_MONTGOMERY = 0, 1   # csg.h: representation of the trace words crossing the boundary
 TRACE_WIDTH = {AIR_TRANSACTION: 94, AIR_MERKLE_UPDATE: 65, AIR_MERKLE_INIT: 58, AIR_SCHNORR: 56, AIR_RANGE: 2, AIR_RESCUE: 14}
+NUM_CONSTRAINTS = {AIR_TRANSACTION: 115, AIR_MERKLE_UPDATE: 106, AIR_MERKLE_INIT: 56, AIR_SCHNORR: 56, AIR_RANGE: 2, AIR_RESCUE: 14}
+REPORT_CAP = 256   # csg.h CSG_REPORT_CAP
 _ERRORS = {1: "invalid argument", 2: "CUDA error", 3: "call out of order", 4: "unsupported", 5: "random coin failure"}
 
 
@@ -58,6 +60,29 @@ class Timings(C.Structure):
         d = {n: getattr(self, n) for n, _ in self._fields_ if n != "stage_launches"}
         d["stage_launches"] = dict(zip(self.STAGES, [int(v) for v in self.stage_launches]))
         return d
+
+
+class TraceReport(C.Structure):
+    """csg_trace_report: the verdict of csg_validate_* on one trace (winterfell's debug-build trace.validate)"""
+    _fields_ = [("failed_steps", C.c_uint64), ("failed_cells", C.c_uint64), ("num_transition", C.c_uint32), ("num_boundary", C.c_uint32),
+                ("_transition", C.c_uint32 * 2 * REPORT_CAP), ("_boundary", C.c_uint32 * 2 * REPORT_CAP)]
+
+    @property
+    def ok(self) -> bool:
+        return self.failed_steps == 0 and self.failed_cells == 0
+
+    @property
+    def transition(self) -> list:
+        """(step, constraint) of the first REPORT_CAP non-zero transition constraints, ascending"""
+        return [(int(self._transition[i][0]), int(self._transition[i][1])) for i in range(self.num_transition)]
+
+    @property
+    def boundary(self) -> list:
+        """(column, step) of the first REPORT_CAP failing asserted cells, ascending by step, then column"""
+        return [(int(self._boundary[i][0]), int(self._boundary[i][1])) for i in range(self.num_boundary)]
+
+    def __repr__(self):
+        return f"TraceReport(failed_steps={self.failed_steps}, failed_cells={self.failed_cells}, transition={self.transition[:4]}..., boundary={self.boundary[:4]}...)"
 
 
 def build(force: bool = False) -> Path:
@@ -106,6 +131,10 @@ def lib() -> C.CDLL:
         "csg_open_trace": (C.c_int, [vp, _u64p, C.c_size_t, _u64p, _u8p, C.c_size_t, _szp]),
         "csg_open_composition": (C.c_int, [vp, _u64p, C.c_size_t, _u64p, _u8p, C.c_size_t, _szp]),
         "csg_open_fri_layer": (C.c_int, [vp, C.c_size_t, _u64p, C.c_size_t, _u64p, _u8p, C.c_size_t, _szp]),
+        "csg_validate_trace": (C.c_int, [vp, C.c_int, _u64p, C.c_int, C.c_size_t, _u64p, C.c_size_t, C.POINTER(TraceReport)]),
+        "csg_validate_resident_trace": (C.c_int, [vp, C.POINTER(TraceReport)]),
+        "csg_validate_many_device": (C.c_int, [vp, C.c_int, C.c_size_t, vp, C.c_int, C.c_size_t, _u64p, C.c_size_t, C.POINTER(TraceReport)]),
+        "csg_debug_transition_at": (C.c_int, [C.c_int, C.c_size_t, _u64p, C.c_size_t, C.c_size_t, _u64p, _u64p, _u64p]),
         "csg_verify": (C.c_int, [C.c_int, _u64p, C.c_size_t, _u8p, C.c_size_t]),
         "csg_verify_with_options": (C.c_int, [C.c_int, _u64p, C.c_size_t, _u8p, C.c_size_t, opt]),
         "csg_get_timings": (C.c_int, [vp, C.POINTER(Timings)]),
@@ -160,6 +189,19 @@ def verify(air_id: int, pub: np.ndarray, proof: bytes, min_options: "ProofOption
     if min_options is not None:
         return lib().csg_verify_with_options(air_id, _p64(pub), pub.size, _p8(buf), buf.size, C.byref(min_options))
     return lib().csg_verify(air_id, _p64(pub), pub.size, _p8(buf), buf.size)
+
+
+def debug_transition_at(air_id: int, trace_len: int, pub, step: int, cur, nxt) -> np.ndarray:
+    """csg_debug_transition_at: every transition constraint slot of the AIR at `step` on rows cur, nxt (canonical words); host-only"""
+    pub = np.ascontiguousarray(pub, dtype=np.uint64)
+    cur, nxt = np.ascontiguousarray(cur, dtype=np.uint64), np.ascontiguousarray(nxt, dtype=np.uint64)
+    if cur.shape != (TRACE_WIDTH[air_id],) or nxt.shape != cur.shape:
+        raise CsgError(f"rows of {TRACE_WIDTH[air_id]} words expected")
+    out = np.zeros(NUM_CONSTRAINTS[air_id], dtype=np.uint64)
+    rc = lib().csg_debug_transition_at(air_id, trace_len, _p64(pub), pub.size, step, _p64(cur), _p64(nxt), _p64(out))
+    if rc:
+        raise CsgError(f"{_ERRORS.get(rc, rc)}: csg_debug_transition_at")
+    return out
 
 
 class Context:
@@ -307,6 +349,40 @@ class Context:
         out, pubs = self._device_traces(batch.num_tx, 94, 1024), np.zeros((batch.num_tx, 14), dtype=np.uint64)
         self._check(lib().csg_build_traces_many_transaction(self._h, batch._h, out.data_ptr(), _p64(pubs)))
         return out, pubs
+
+    # ---- trace validation: winterfell's debug-build trace.validate(&air), on the GPU (csg_validate_*)
+    def validate(self, air_id: int, trace: np.ndarray, pub: np.ndarray, repr: int = REPR_CANONICAL) -> TraceReport:
+        """csg_validate_trace: check a (width, n) HOST trace (pageable, or a HostBuffer's array) against its AIR"""
+        trace = np.ascontiguousarray(trace, dtype=np.uint64)
+        pub = np.ascontiguousarray(pub, dtype=np.uint64)
+        if trace.ndim != 2 or trace.shape[0] != TRACE_WIDTH[air_id]:
+            raise CsgError(f"trace must be ({TRACE_WIDTH[air_id]}, n)")
+        r = TraceReport()
+        self._check(lib().csg_validate_trace(self._h, air_id, _p64(trace), repr, trace.shape[1], _p64(pub), pub.size, C.byref(r)))
+        return r
+
+    def validate_resident(self) -> TraceReport:
+        """csg_validate_resident_trace: check the trace prove_loaded would prove"""
+        r = TraceReport()
+        self._check(lib().csg_validate_resident_trace(self._h, C.byref(r)))
+        return r
+
+    def validate_many_device(self, air_id: int, traces, pubs, repr: int = REPR_CANONICAL) -> list:
+        """csg_validate_many_device: one TraceReport per trace of a contiguous int64 / uint64 torch CUDA tensor (K, width, n) on this
+        context's device, read in place.  Torch's current stream is synchronised first, as in prove_many_device."""
+        import torch
+        if not isinstance(traces, torch.Tensor) or traces.device.type != "cuda":
+            raise CsgError("traces must be a torch CUDA tensor (K, width, n)")
+        if traces.dtype not in (torch.int64, torch.uint64) or not traces.is_contiguous():
+            raise CsgError("traces must be a contiguous int64 or uint64 tensor")
+        if traces.ndim != 3 or traces.shape[1] != TRACE_WIDTH[air_id]:
+            raise CsgError(f"traces must be (K, {TRACE_WIDTH[air_id]}, n)")
+        k = traces.shape[0]
+        pubs = np.ascontiguousarray(pubs, dtype=np.uint64).reshape(k, -1)
+        torch.cuda.current_stream(traces.device).synchronize()
+        out = (TraceReport * max(k, 1))()
+        self._check(lib().csg_validate_many_device(self._h, air_id, k, traces.data_ptr(), repr, traces.shape[2], _p64(pubs), pubs.shape[1], out))
+        return [out[i] for i in range(k)]
 
     def prove_columns(self, air_id: int, columns, pub: np.ndarray, options: ProofOptions, repr: int = REPR_CANONICAL) -> bytes:
         """csg_prove_columns: one separately allocated array per trace column (how a winterfell TraceTable holds them)"""

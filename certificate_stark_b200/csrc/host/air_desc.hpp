@@ -56,4 +56,9 @@ struct BoundaryGroups {
 TransitionGroups transition_groups(const AirDesc &air);
 BoundaryGroups boundary_groups(const AirDesc &air);
 
+// the merged transition constraints sum_s result_s * (alpha_s + beta_s * xp[group(s)]) of AIR `id` on one row pair, host build of
+// airs.cuh (verifier.cpp); pv: the periodic values of the row.  With a one-hot alpha and beta = 0 it is result_s alone.
+fe eval_merged_any(int id, const AirDesc &air, const TransitionGroups &tg, const std::vector<fe> &cur, const std::vector<fe> &next, const std::vector<fe> &pv,
+                   const std::vector<fe> &alpha, const std::vector<fe> &beta, const std::vector<fe> &xp);
+
 }  // namespace csg

@@ -18,6 +18,36 @@ namespace csg {
 using namespace f63;
 
 namespace {
+template <int AIR>
+fe eval_merged(const AirDesc &air, const TransitionGroups &tg, const std::vector<fe> &cur, const std::vector<fe> &next, const std::vector<fe> &pv,
+               const std::vector<fe> &alpha, const std::vector<fe> &beta, const std::vector<fe> &xp) {
+    const size_t w = air.width, np = pv.size();
+    std::vector<fe> m(2 * w);
+    for (size_t c = 0; c < w; c++) { m[2 * c] = cur[c]; m[2 * c + 1] = next[c]; }
+    std::vector<uint32_t> off(np + 1), mask(np + 1, 0);
+    for (size_t c = 0; c <= np; c++) off[c] = (uint32_t)c;
+    std::vector<fe> pvp(pv); pvp.push_back(0);
+    airs::Frame f{m.data(), m.data() + 1, 2};
+    airs::Periodic Pv{pvp.data(), off.data(), mask.data(), 0};
+    airs::Comb C{alpha.data(), beta.data(), tg.group_of.data(), xp.data(), 1, acc192(), nullptr, 0};
+    airs::eval_transition<AIR>(f, Pv, C);
+    return C.sum.reduce();
+}
+}  // namespace
+// declared in air_desc.hpp: also the host side of trace validation (validate/)
+fe eval_merged_any(int id, const AirDesc &air, const TransitionGroups &tg, const std::vector<fe> &cur, const std::vector<fe> &next, const std::vector<fe> &pv,
+                   const std::vector<fe> &alpha, const std::vector<fe> &beta, const std::vector<fe> &xp) {
+    switch (id) {
+    case 0: return eval_merged<0>(air, tg, cur, next, pv, alpha, beta, xp);
+    case 1: return eval_merged<1>(air, tg, cur, next, pv, alpha, beta, xp);
+    case 2: return eval_merged<2>(air, tg, cur, next, pv, alpha, beta, xp);
+    case 3: return eval_merged<3>(air, tg, cur, next, pv, alpha, beta, xp);
+    case 4: return eval_merged<4>(air, tg, cur, next, pv, alpha, beta, xp);
+    default: return eval_merged<5>(air, tg, cur, next, pv, alpha, beta, xp);
+    }
+}
+
+namespace {
 
 struct Reader {
     const uint8_t *p; size_t len, off = 0; bool bad = false;
@@ -112,32 +142,6 @@ bool batch_opening_root(int hash_fn, const uint8_t *paths, size_t plen, const st
     return true;
 }
 
-template <int AIR>
-fe eval_merged(const AirDesc &air, const TransitionGroups &tg, const std::vector<fe> &cur, const std::vector<fe> &next, const std::vector<fe> &pv,
-               const std::vector<fe> &alpha, const std::vector<fe> &beta, const std::vector<fe> &xp) {
-    const size_t w = air.width, np = pv.size();
-    std::vector<fe> m(2 * w);
-    for (size_t c = 0; c < w; c++) { m[2 * c] = cur[c]; m[2 * c + 1] = next[c]; }
-    std::vector<uint32_t> off(np + 1), mask(np + 1, 0);
-    for (size_t c = 0; c <= np; c++) off[c] = (uint32_t)c;
-    std::vector<fe> pvp(pv); pvp.push_back(0);
-    airs::Frame f{m.data(), m.data() + 1, 2};
-    airs::Periodic Pv{pvp.data(), off.data(), mask.data(), 0};
-    airs::Comb C{alpha.data(), beta.data(), tg.group_of.data(), xp.data(), 1, acc192(), nullptr, 0};
-    airs::eval_transition<AIR>(f, Pv, C);
-    return C.sum.reduce();
-}
-fe eval_merged_any(int id, const AirDesc &air, const TransitionGroups &tg, const std::vector<fe> &cur, const std::vector<fe> &next, const std::vector<fe> &pv,
-                   const std::vector<fe> &alpha, const std::vector<fe> &beta, const std::vector<fe> &xp) {
-    switch (id) {
-    case 0: return eval_merged<0>(air, tg, cur, next, pv, alpha, beta, xp);
-    case 1: return eval_merged<1>(air, tg, cur, next, pv, alpha, beta, xp);
-    case 2: return eval_merged<2>(air, tg, cur, next, pv, alpha, beta, xp);
-    case 3: return eval_merged<3>(air, tg, cur, next, pv, alpha, beta, xp);
-    case 4: return eval_merged<4>(air, tg, cur, next, pv, alpha, beta, xp);
-    default: return eval_merged<5>(air, tg, cur, next, pv, alpha, beta, xp);
-    }
-}
 xe fold_row(int d, const xe v[4], fe x_inv, const xe &alpha, fe zeta_inv, fe quarter) {
     xe s02 = x_add(v[0], v[2]), d02 = x_sub(v[0], v[2]), s13 = x_add(v[1], v[3]), d13 = x_scale(x_sub(v[1], v[3]), zeta_inv);
     xe c[4] = {x_add(s02, s13), x_add(d02, d13), x_sub(s02, s13), x_sub(d02, d13)};

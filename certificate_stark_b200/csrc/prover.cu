@@ -30,6 +30,7 @@ void csg_destroy(csg_ctx *ctx) {
     for (auto e : ctx->stage_ev) if (e) cudaEventDestroy(e);
     if (ctx->h2d_a) { cudaEventDestroy(ctx->h2d_a); cudaEventDestroy(ctx->h2d_b); }
     many_delete(ctx->many);
+    validator_delete(ctx->validator);
     delete ctx;
     cudaStreamDestroy(s);
 }

@@ -30,6 +30,7 @@
 #include "many/many.cuh"
 #include "ntt.cuh"
 #include "stages.cuh"
+#include "validate/validate.cuh"
 #include "witness.cuh"
 
 
@@ -238,6 +239,7 @@ struct csg_ctx {
     cudaEvent_t h2d_a = nullptr, h2d_b = nullptr;   // first byte .. last byte of the overlapped H2D copy, on the copy stream
     CosetTables lde_tables;                      // per-coset scale tables of the LDE domain, built once per csg_set_air
     ManyProver *many = nullptr;                  // csg_prove_many: its own device buffers and tables, created by the first batch
+    Validator *validator = nullptr;              // csg_validate_*: its own device buffers, created by the first call
 
     // ------------------------------------------------------------------------------------------ setup
     void set_air(int air_id, size_t trace_len, const csg_options *o, const uint64_t *pub, size_t npub) {

@@ -15,7 +15,8 @@
  * plus the witness builders (build_trace of each prover) and a few kernel-level entry points used by the
  * parity tests and the kernel sweep.  All functions return 0 on success; they never unwind.  A context is
  * single-threaded and owns all device memory; every pointer argument is a HOST pointer owned by the caller, except the
- * traces_dev buffers of csg_prove_many_device and csg_build_traces_many_*, which are device memory the caller owns.
+ * traces_dev buffers of csg_prove_many_device, csg_validate_many_device and csg_build_traces_many_*, which are device memory the
+ * caller owns.
  */
 #ifndef CSG_H
 #define CSG_H
@@ -109,6 +110,40 @@ int csg_prove_many(csg_ctx *ctx, int air_id, size_t count, const uint64_t *const
  * stream that wrote it): the batch runs on the context's own stream. */
 int csg_prove_many_device(csg_ctx *ctx, int air_id, size_t count, const uint64_t *traces_dev, int repr, size_t trace_len,
                           const uint64_t *pubs, size_t npub, const csg_options *opt, uint8_t **proofs, size_t *proof_lens);
+/* ---- trace validation: winterfell's debug-build check `trace.validate(&air)` before Prover::prove, on the GPU ---------------
+ * Every transition constraint is evaluated at every step s in [0, n-1) on rows (s, s+1), and every asserted cell of the AIR's
+ * assertions (single, periodic and sequence) is compared with its value.  A word >= p counts as its residue, as in csg_prove.
+ * The report carries the verdict: a valid trace and an invalid one both return CSG_OK; error codes mean the call itself failed.
+ * A step is flagged when either of two independent random combinations of its constraint values is non-zero (a failing step is
+ * missed with probability about 2^-123); the host then evaluates every constraint of the first flagged steps one by one.
+ * The calls leave the context's single-proof state (csg_set_air, the resident and the prefetched trace) and the csg_prove_many
+ * batch alone; their device buffers are grow-only and freed by csg_destroy.  A context attached to a group (world > 1) gets
+ * CSG_ERR_UNSUPPORTED. */
+enum { CSG_REPORT_CAP = 256 };
+typedef struct {
+    uint64_t failed_steps;                   /* steps s in [0, n-1) where some transition constraint of (row s, row s+1) is non-zero */
+    uint64_t failed_cells;                   /* asserted cells (column, step) whose word differs from the assertion's value */
+    uint32_t num_transition, num_boundary;   /* entries used below */
+    uint32_t transition[CSG_REPORT_CAP][2];  /* (step, constraint): the first CSG_REPORT_CAP non-zero pairs, ascending; constraint =
+                                                the reference's result[] slot */
+    uint32_t boundary[CSG_REPORT_CAP][2];    /* (column, step): the first CSG_REPORT_CAP failing cells, ascending by step, then column */
+} csg_trace_report;
+/* a host trace in csg_prove's layout and representations (pageable or page-locked memory); trace_len up to 2^22 */
+int csg_validate_trace(csg_ctx *ctx, int air_id, const uint64_t *trace, int repr, size_t trace_len, const uint64_t *pub, size_t npub,
+                       csg_trace_report *out);
+/* the trace csg_prove_loaded would prove, for the AIR of csg_set_air (csg_load_trace, csg_build_trace_*_device,
+ * csg_build_trace_transaction_resident); CSG_ERR_STATE when there is none */
+int csg_validate_resident_trace(csg_ctx *ctx, csg_trace_report *out);
+/* count traces in ONE device buffer [count][width][trace_len], read in place and never written; the checks and limits of
+ * csg_prove_many_device (count 1..1024, count * width <= 65535, trace_len <= 2^16, device memory of the context's device).
+ * out receives count reports, report k that of trace k (pubs + k * npub). */
+int csg_validate_many_device(csg_ctx *ctx, int air_id, size_t count, const uint64_t *traces_dev, int repr, size_t trace_len,
+                             const uint64_t *pubs, size_t npub, csg_trace_report *out);
+/* debugging aid, host-only (no context, no GPU): the value of every transition constraint slot of the AIR at one step, canonical.
+ * cur / next: the rows s and s+1 as canonical words (width each); out: one word per constraint. */
+int csg_debug_transition_at(int air_id, size_t trace_len, const uint64_t *pub, size_t npub, size_t step, const uint64_t *cur,
+                            const uint64_t *next, uint64_t *out);
+
 /* ---- verification: replaces `winterfell::verify::<Air>(proof, pub_inputs)` (src/lib.rs:144-150).  Host-only, as in the
  * reference; needs no context and no GPU.  Returns CSG_OK or one of CSG_VERIFY_*. */
 int csg_verify(int air_id, const uint64_t *pub, size_t npub, const uint8_t *proof, size_t proof_len);
