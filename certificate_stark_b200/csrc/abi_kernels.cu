@@ -3,7 +3,6 @@
 
 extern "C" {
 
-// 3 = merged constraint column, 4 = composition columns, 5 = composition LDE)
 long long csg_debug_redc_violations(csg_ctx *) { return (long long)redc_violations(); }
 long long csg_debug_redc_selftest(csg_ctx *ctx) {
     long long bad = -1;
@@ -15,14 +14,22 @@ long long csg_debug_field_selftest(csg_ctx *ctx) {
     guarded(ctx, [&] { bad = field_selftest(ctx->st); });
     return bad;
 }
+// words >= p in stage buffer `which` (0 = trace coefficients, 1 = trace LDE, 2 = periodic tables, 3 = merged constraint column,
+// 4 = composition columns, 5 = composition LDE), all `ext` planes of 3-5; -1 for another `which` or an error.  The copy runs on
+// the proving stream, after the work queued there that writes the buffer.
 long long csg_debug_count_unreduced(csg_ctx *ctx, int which) {
+    if (which < 0 || which > 5) return -1;
     long long bad = -1;
     guarded(ctx, [&] {
         const DBuf<fe> *b = which == 0 ? &ctx->d_polys : which == 1 ? &ctx->d_lde : which == 2 ? &ctx->d_ptab : which == 3 ? &ctx->d_comb : which == 4 ? &ctx->d_cpolys : &ctx->d_clde;
-        size_t count = which == 0 ? ctx->air.width * ctx->n : which == 1 ? ctx->air.width * ctx->lde_n : which == 2 ? ctx->h_cargs->ptab_coset_stride * ctx->ce
-                       : which == 3 ? ctx->ce * ctx->n : which == 4 ? ctx->ce * ctx->n : ctx->ce * ctx->lde_n;
+        const size_t d = (size_t)ctx->d, cel = ctx->cel;
+        size_t count = which == 0 ? ctx->air.width * ctx->n : which == 1 ? ctx->air.width * ctx->n * ctx->bl
+                       : which == 2 ? (ctx->h_cargs ? ctx->h_cargs->ptab_coset_stride * cel : 0)
+                       : which == 3 ? d * cel * ctx->n : which == 4 ? d * ctx->ce * ctx->n : d * ctx->ce * ctx->n * ctx->bl;
+        count = std::min(count, b->n);   // a stage that has not run yet has not sized its buffer
         std::vector<fe> h(count);
-        CSG_CUDA(cudaMemcpy(h.data(), b->p, count * sizeof(fe), cudaMemcpyDeviceToHost));
+        if (count) CSG_CUDA(cudaMemcpyAsync(h.data(), b->p, count * sizeof(fe), cudaMemcpyDeviceToHost, ctx->st.s));
+        CSG_CUDA(cudaStreamSynchronize(ctx->st.s));
         bad = 0;
         for (fe v : h) bad += v >= P;
     });
